@@ -7,6 +7,7 @@ Workload (BASELINE.json `metric`): 100 000 UEs x 4096 replications per GPU, Beta
 step (= one pass of the hot path over the batch) is 8.192e11 updates per GPU.
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            our arm (CUDA, librach_gpu)
+    python bench.py ... --dump-outputs DIR                         also write the last step's outputs as DIR/*.npy
     python bench.py --impl reference [--steps K] [--warmup W]      the reference's own CPU code
 
 One JSON line on stdout (rank 0).  See DESIGN.md section 6 for what each key means.
@@ -195,6 +196,29 @@ def full_replication_pair(pkg, device, procs):
 
 
 # ------------------------------------------------------------------------------------------------
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_SKIP = ("updates", "recordMoves")      # engine work counters: how the engine scheduled its work, not results
+
+
+def dump_outputs(out_dir, st, suffix="", limit=DUMP_LIMIT_BYTES):
+    """What the last timed step returned to its caller: the per-replication counters of the simulation
+    (ra_sim_stats_all), one float64 array per counter, indexed [point, replication] -- 11 x 4096 x 8 B at the headline
+    size.  Above `limit` bytes a fixed, seeded sample of replications is written, and replication.npy holds their
+    indices.  Two builds run with the same arguments see the same inputs (seeded tape, fixed replication ids), so
+    their files compare value for value."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    names = [n for n in st.dtype.names if n not in DUMP_SKIP]
+    reps = st.shape[1]
+    keep = max(1, min(reps, limit // (8 * len(names) * st.shape[0] + 8)))
+    if keep < reps:
+        idx = np.sort(np.random.default_rng(0).choice(reps, keep, replace=False))
+        st = st[:, idx]
+        np.save(os.path.join(out_dir, "replication" + suffix + ".npy"), idx.astype(np.float64))
+    for name in names:
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), st[name].astype(np.float64))
+
+
 def run_our_arm(args):
     import torch
     import torch.distributed as dist
@@ -238,6 +262,8 @@ def run_our_arm(args):
 
     st = sim.stats_all()
     stats_bytes = st.nbytes
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, st, "_rank%d" % rank if world > 1 else "", DUMP_LIMIT_BYTES // world)
     t = torch.tensor([kernel_ms, wall_ms], dtype=torch.float64, device="cuda")
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)            # max over ranks of the device time
@@ -320,7 +346,15 @@ def main():
     ap.add_argument("--ctas-per-sm", type=int, default=0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-full-replication", action="store_true", help="skip the ~1-2 min complete-replication CPU/GPU pair")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's per-replication counters to DIR/<counter>.npy (float64, at most "
+                         "64 MB: a seeded sample of replications above that); with several ranks each writes "
+                         "DIR/<counter>_rank<r>.npy.  bench_outputs/ is git-ignored")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU arm's outputs (--impl ours)")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

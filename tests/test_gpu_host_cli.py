@@ -1,6 +1,8 @@
 """The C host program (5g-nr-randomaccess_b200/host/rach_sim.c) against the reference's own
 stdout report and result files (RandomAccessWithNOMA.c:354-361, 741-825) produced by the
-tape-mode reference build -- byte for byte."""
+tape-mode reference build -- byte for byte where that build exists (oracle/_ref), and always against a
+stored digest of the host program's reports on the same runs (tests/golden/recorded_outputs.json; how it was
+recorded: tests/conftest.py, Recorded)."""
 import importlib
 import os
 import subprocess
@@ -21,6 +23,15 @@ O.run_ref("w", cfg, per_ue=False)
 ''' % ROOT
 
 
+def _outputs(args, out, d):
+    """One run of the host program: its arguments, its stdout and every file it wrote under d."""
+    got = {"args": args, "stdout": out}
+    for f in sorted(d.rglob("*")):
+        if f.is_file():
+            got[str(f.relative_to(d))] = f.read_bytes()
+    return got
+
+
 def _reference(tmp, nue, rep, retx, grant, dist):
     d = tmp / ("ref_%d_%d" % (nue, rep))
     (d / "NomaBetaResults").mkdir(parents=True)
@@ -31,15 +42,16 @@ def _reference(tmp, nue, rep, retx, grant, dist):
 
 
 @pytest.mark.parametrize("dist,sub", [(0, "NomaBetaResults"), (1, "NomaUniformResults")])
-def test_stdout_and_files_match_reference(tmp_path, oracle, dist, sub):
-    if not oracle.ref_available("w"):
-        pytest.skip("oracle/_ref not shipped")
+def test_stdout_and_files_match_reference(tmp_path, oracle, recorded, dist, sub):
     pkg = importlib.import_module("5g-nr-randomaccess_b200")
     exe = pkg.build_host()
     nues, retx, grant = [1500, 4000], 5, 7
-    out = subprocess.run([exe, "-t", "2", "-d", str(dist), "-mrc", str(retx), "-g", str(grant), "--nue",
-                          ",".join(map(str, nues)), "--outdir", str(tmp_path / "ours")],
+    args = ["-t", "2", "-d", str(dist), "-mrc", str(retx), "-g", str(grant), "--nue", ",".join(map(str, nues))]
+    out = subprocess.run([exe] + args + ["--outdir", str(tmp_path / "ours")],
                          capture_output=True, text=True, check=True).stdout
+    recorded.check("cli_w_" + sub, recorded.digest(**_outputs(args, out, tmp_path / "ours")))
+    if not oracle.ref_available("w"):
+        return
     blocks = out.split("-------- ")
     assert blocks[0] == ("Traffic model: Uniform\n\n" if dist == 1 else "Traffic model: Beta\n\n")
     k = 1
@@ -89,16 +101,24 @@ def _strip_latency(text):
 
 
 @pytest.mark.parametrize("dist,sub", [(0, "BasicBetaSimulationResults"), (1, "BasicUniformSimulationResults")])
-def test_format_b_matches_randomaccesssimulatorbeta(tmp_path, oracle, dist, sub):
+def test_format_b_matches_randomaccesssimulatorbeta(tmp_path, oracle, recorded, dist, sub):
     """--format b: stdout block (B:200-209, 440-446) and files (B:460-482, 484-514) of RandomAccessSimulatorBeta.c;
     the clock() latency line / 6th file line is the only thing not compared."""
-    if not oracle.ref_available("b"):
-        pytest.skip("oracle/_ref not shipped")
     pkg = importlib.import_module("5g-nr-randomaccess_b200")
     exe = pkg.build_host()
     nue = 3000
-    out = subprocess.run([exe, "--format", "b", "-t", "2", "-d", str(dist), "--nue", str(nue), "--outdir", str(tmp_path / "ours")],
+    args = ["--format", "b", "-t", "2", "-d", str(dist), "--nue", str(nue)]
+    out = subprocess.run([exe] + args + ["--outdir", str(tmp_path / "ours")],
                          capture_output=True, text=True, check=True).stdout
+    got = _outputs(args, _strip_latency(out), tmp_path / "ours")
+    for name in got:
+        if name.endswith("_Results.txt"):
+            lines = got[name].split(b"\n")
+            assert len(lines) == 6, name
+            got[name] = b"\n".join(lines[:5])
+    recorded.check("cli_b_" + sub, recorded.digest(**got))
+    if not oracle.ref_available("b"):
+        return
     blocks = out.split("-------- ")
     for seed in (0, 1):
         d = tmp_path / ("refb_%d" % seed)
@@ -118,15 +138,17 @@ def test_format_b_matches_randomaccesssimulatorbeta(tmp_path, oracle, dist, sub)
         assert ours_log == ref_log, seed
 
 
-def test_format_n_matches_noma_c(tmp_path, oracle):
+def test_format_n_matches_noma_c(tmp_path, oracle, recorded):
     """--format n: NOMA.c's result line (N:598-635) on stdout and appended to TestResults/Sector_<nUE>_Result.txt."""
-    if not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "libref_n.so")):
-        pytest.skip("oracle/_ref/libref_n.so not shipped")
     pkg = importlib.import_module("5g-nr-randomaccess_b200")
     exe = pkg.build_host()
     nues = [2000, 6000]
-    out = subprocess.run([exe, "--format", "n", "-t", "2", "--nue", ",".join(map(str, nues)), "--outdir", str(tmp_path / "ours")],
+    args = ["--format", "n", "-t", "2", "--nue", ",".join(map(str, nues))]
+    out = subprocess.run([exe] + args + ["--outdir", str(tmp_path / "ours")],
                          capture_output=True, text=True, check=True).stdout
+    recorded.check("cli_n", recorded.digest(**_outputs(args, out, tmp_path / "ours")))
+    if not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "libref_n.so")):
+        return
     exp = ""
     files = {n: "" for n in nues}
     for seed in (0, 1):
@@ -154,19 +176,21 @@ print("COUNTERS %%d %%d %%d %%d" %% (r.collisionPreambles, r.totalPreambleTxop, 
 ''' % ROOT
 
 
-def test_format_u_matches_random_access_simulator_c(tmp_path, oracle):
+def test_format_u_matches_random_access_simulator_c(tmp_path, oracle, recorded):
     """--format u: the report of RandomAccessSimulator.c (U0:69-70, 141-143, 277-345): stdout, *_Results.txt and
     *_Logs.txt byte for byte against the tape-mode build of that file; its collision / tx-opportunity counters are
     globals that accumulate over the nUE sweep (U0:36-37), so the second point's two ratio lines are checked
     against the sums."""
     import numpy as np
-    if not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "libref_u0.so")):
-        pytest.skip("oracle/_ref/libref_u0.so not shipped")
     pkg = importlib.import_module("5g-nr-randomaccess_b200")
     exe = pkg.build_host()
     nues = [20000, 30000]
-    out = subprocess.run([exe, "--format", "u", "--nue", ",".join(map(str, nues)), "--outdir", str(tmp_path / "ours")],
+    args = ["--format", "u", "--nue", ",".join(map(str, nues))]
+    out = subprocess.run([exe] + args + ["--outdir", str(tmp_path / "ours")],
                          capture_output=True, text=True, check=True).stdout
+    recorded.check("cli_u", recorded.digest(**_outputs(args, out, tmp_path / "ours")))
+    if not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "libref_u0.so")):
+        return
     refs = []
     for n in nues:
         d = tmp_path / ("refu_%d" % n)

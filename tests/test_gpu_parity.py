@@ -146,12 +146,15 @@ def test_shape_follows_the_job_count(pkg, oracle):
         assert (st == ref[:reps]).all(), reps
 
 
-def test_against_reference_sources_in_tape_mode(pkg, oracle):
-    if not oracle.ref_available("w"):
-        pytest.skip("oracle/_ref not shipped")
+def test_against_reference_sources_in_tape_mode(pkg, oracle, recorded):
+    """Against the tape-mode reference build where it exists, and always against the stored digest of the engine's
+    output on the same case (how it was recorded: tests/conftest.py, Recorded)."""
     kw = dict(nUE=8000, seed=31, rep=17)
-    r, ue_ref, _ = oracle.run_ref("w", oracle.make_config(**kw))
     st, ue, _ = _run_gpu(pkg, kw)
+    recorded.check("gpu_tape_mode_w", recorded.digest(config=kw, ue=ue, **{k: getattr(st, k) for k in KEYS[:8]}))
+    if not oracle.ref_available("w"):
+        return
+    r, ue_ref, _ = oracle.run_ref("w", oracle.make_config(**kw))
     for k in KEYS[:8]:
         assert getattr(st, k) == getattr(r, k), k
     np.testing.assert_array_equal(ue, ue_ref)
