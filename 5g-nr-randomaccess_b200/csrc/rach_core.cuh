@@ -112,49 +112,9 @@ RA_HD unsigned ra_mod(unsigned x, unsigned d, unsigned magic, unsigned shift) {
 /* A calendar record is written once and read once, several ms later, by which time a thousand other replications have been
  * through the caches: streaming (evict-first) stores and loads keep the 16-byte records from displacing what IS re-used
  * (work lists, position hints).  Measured on the bench workload: 965 -> 945 ms. */
-/* tuning switches of the mover path (A/B timings in profiles/r02j_*) */
-#ifndef RA_IDX32
-#define RA_IDX32 1          /* 32-bit record index into the move calendar */
-#endif
-#ifndef RA_ALIGN_CLOSED
-#define RA_ALIGN_CLOSED 1   /* branch-free slot alignment for a compile-time subframe */
-#endif
-#ifndef RA_LIGHT_ROWSKIP
-#define RA_LIGHT_ROWSKIP 0  /* 1: the class view of a light ms reads only the cohorts of the window that hold a live record (measured 1-2 % slower than the straight-line loads of all rows) */
-#endif
-#ifndef RA_P5_RANK
-#define RA_P5_RANK 1        /* phase 5: rank by counting when a ms has at most 32 singleton scans */
-#endif
-#ifndef RA_MIN_PLAIN_FIRST
-#define RA_MIN_PLAIN_FIRST 0   /* 1: read the cohort minimum first and only then atomicMin (measured 0.6 % slower than the bare atomic) */
-#endif
-#ifndef RA_LD_HINT
-#define RA_LD_HINT 1        /* 0 plain, 1 ld.global.cs (streaming), 2 ld.global.lu (last use) */
-#endif
-#ifndef RA_ST_HINT
-#define RA_ST_HINT 1        /* 0 plain, 1 st.global.cs (streaming), 2 st.global.cg, 3 st.global.wt */
-#endif
 #ifdef __CUDA_ARCH__
-__device__ __forceinline__ ::uint4 ra_ldrec(const ::uint4* p) {
-#if RA_LD_HINT == 1
-    return __ldcs(p);
-#elif RA_LD_HINT == 2
-    return __ldlu(p);
-#else
-    return *p;
-#endif
-}
-__device__ __forceinline__ void ra_strec(::uint4* p, const ::uint4& v) {
-#if RA_ST_HINT == 1
-    __stcs(p, v);
-#elif RA_ST_HINT == 2
-    __stcg(p, v);
-#elif RA_ST_HINT == 3
-    __stwt(p, v);
-#else
-    *p = v;
-#endif
-}
+__device__ __forceinline__ ::uint4 ra_ldrec(const ::uint4* p) { return __ldcs(p); }
+__device__ __forceinline__ void ra_strec(::uint4* p, const ::uint4& v) { __stcs(p, v); }
 #define RA_STREC(p, v) ra_strec((p), (v))
 #define RA_LDREC(p)    ra_ldrec(p)
 #else
@@ -312,15 +272,8 @@ RA_HD int ra_align_pt(const PT& pt, int subTime) {
  * multiply-shift division, no branch (r == 0 -> +1, r == 1 -> +0, else +(A - r + 1), all of them A * floor((subTime + A - 2) / A) + 1) */
 template <int P_, int BI_, int A_, int Wn_, int R_>
 RA_HD int ra_align_pt(const RaPointFixed<P_, BI_, A_, Wn_, R_>&, int subTime) {
-#if RA_ALIGN_CLOSED
     if (A_ >= 2) return (int)(((unsigned)subTime + (unsigned)(A_ - 2)) / (unsigned)A_ * (unsigned)A_) + 1;
     return subTime + 1;
-#else
-    const int r = (int)((unsigned)subTime % (unsigned)A_);
-    if (r == 0) return subTime + 1;
-    if (r == 1) return subTime;
-    return subTime + (A_ - r + 1);
-#endif
 }
 
 template <class PT>
@@ -402,11 +355,7 @@ RA_HD unsigned ra_bucket_push(const PT& pt, const RaWork& w, RaShared& s, int m,
      * per bucket with __match_any_sync (the variable-mask shuffle that follows costs more than the contention) */
     unsigned pos = RA_AADD(&S_bcount[slot], 1u);
     if (pos >= (unsigned)w.cap) { s.overflow = 1; return 0; }
-#if RA_IDX32
     RA_STREC(&w.bucket[slot * (unsigned)w.cap + pos], rec);      /* ring x capacity < 2^32 records (checked at create) */
-#else
-    RA_STREC(&w.bucket[(size_t)slot * w.cap + pos], rec);
-#endif
     return pos;
 }
 
@@ -418,13 +367,8 @@ RA_HD void ra_schedule(const PT& pt, const RaWork& w, RaShared& s, const uint4& 
     const unsigned pos = ra_bucket_push(pt, w, s, m, rec);
     unsigned c = ((unsigned)m & (unsigned)(pt.R - 1)) * (unsigned)pt.P + ra_rec_p(rec);
     RA_AADD(&S_cnt[c], 1u);
-#if RA_MIN_PLAIN_FIRST
-    if (rec.x < S_minI[c]) {                              /* plain read first: the minimum rarely moves */
-        if (RA_AMIN(&S_minI[c], rec.x) > rec.x) w.minPos[c] = pos;
-    }
-#else
+    /* a bare atomic: 0.6 % faster than reading the minimum first */
     if (RA_AMIN(&S_minI[c], rec.x) > rec.x) w.minPos[c] = pos;
-#endif
 }
 
 /* a UE whose txTime is not in the future and that nobody postpones (W:516 applied to an old
@@ -858,7 +802,7 @@ __device__ __forceinline__ void ra_phase5_warp(const PT& pt, const RaWork& w, Ra
     unsigned tau = RA_INF32, noGrant = 0;
     if ((long long)n > K) {
         if (K == 0) { noGrant = 1; tau = 0; }
-        else if (RA_P5_RANK && n <= 32u) {
+        else if (n <= 32u) {
             /* at most one singleton per lane (the normal case away from the overload peak, where the singletons of a ms are
              * the UEs of one arrival step -- consecutive indices, all in ONE histogram bin, so the bin walk below would
              * take K full passes): rank by counting, the K-th smallest is the lane whose rank is K - 1 (indices are distinct) */
@@ -1109,8 +1053,7 @@ RW_FN int ra_light_ms(const RaJobT<PT>& job, const RaWork& w, RaShared& s, RaCtl
                 f[l] = 0;
                 if (q < P) {
                     unsigned n = 0, best = RA_INF32, bestm = 0;
-                    for (int d = 1; d < Wn; ++d) {
-                        if (RA_LIGHT_ROWSKIP && canSkip && !((liveSlots >> d) & 1u)) continue;
+                    for (int d = 1; d < Wn; ++d) {      /* all rows: skipping the dead ones measured 1-2 % slower */
                         const unsigned m = ((unsigned)(T + d) & Rm);
                         n += S_cnt[m * P + q];
                         const unsigned v = S_minI[m * P + q]; if (v < best) { best = v; bestm = m; }

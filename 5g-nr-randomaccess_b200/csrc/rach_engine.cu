@@ -57,15 +57,6 @@
                               sector: 192 x 5 169 ms) */
 #endif
 #define RA_NPHASE 10
-#ifndef RA_LIGHT
-#define RA_LIGHT 1           /* 0: every ms takes the general (block-wide) path -- for cross-checks and A/B timing */
-#endif
-#ifndef RA_DEFER
-#define RA_DEFER 1           /* 1: re-transmitters of the ms wait in registers and reach the work list a warp at a time (RaPend) */
-#endif
-#ifndef RA_LOOP_UNROLL
-#define RA_LOOP_UNROLL 1
-#endif
 #ifndef RA_ILP
 #define RA_ILP 2             /* movers per thread and loop iteration (interleaved Philox chains) */
 #endif
@@ -139,21 +130,19 @@ __global__ void __launch_bounds__(NT, MINB) ra_step_kernel(RaKernelArgs a) {
                 else {
                     if (!first) ++T;
                     if (tid == 0) ra_gc_apply(s);
-                    if (RA_LIGHT) {
-                        if (tid == 0) ra_lists_reset(s);
-                        __syncwarp();
-                        RaCtl c = ra_ctl_load(s);
-                        int done = 0;
-                        for (;;) {
-                            code = ra_light_ms<DUMP>(job, w, s, c, &acc, T, &done, &simTime);
-                            if (code != 1) break;
-                            if (done) { code = 4; break; }
-                            ++T;
-                        }
-                        __syncwarp();
-                        if (tid == 0) ra_ctl_store(s, c);
-                        __syncwarp();
+                    if (tid == 0) ra_lists_reset(s);
+                    __syncwarp();
+                    RaCtl c = ra_ctl_load(s);
+                    int done = 0;
+                    for (;;) {
+                        code = ra_light_ms<DUMP>(job, w, s, c, &acc, T, &done, &simTime);
+                        if (code != 1) break;
+                        if (done) { code = 4; break; }
+                        ++T;
                     }
+                    __syncwarp();
+                    if (tid == 0) ra_ctl_store(s, c);
+                    __syncwarp();
                     if (code == 0) ra_phase0(job, s, T, tid, 32);
                     else if (code == 2) ra_phase0_classes(job, s, T, tid, 32);
                 }
@@ -171,7 +160,6 @@ __global__ void __launch_bounds__(NT, MINB) ra_step_kernel(RaKernelArgs a) {
                 const uint4* bT = w.bucket + (size_t)((unsigned)T & (unsigned)(pt.R - 1)) * w.cap;
                 const uint4 dead = make_uint4(RA_DEAD, 0, 0, 0);
                 unsigned i = tid;
-#if RA_ILP >= 2
                 /* the thread walks records tid, tid + NT, ...: one pointer stepped by a compile-time stride (loads at
                  * immediate offsets), `left` = records from the thread's current one to the end of the bucket */
                 const uint4* pr = bT + tid;
@@ -183,9 +171,6 @@ __global__ void __launch_bounds__(NT, MINB) ra_step_kernel(RaKernelArgs a) {
                 uint4 c[RA_ILP];
 #pragma unroll
                 for (int k = 0; k < RA_ILP; ++k) c[k] = left > k * NT ? RA_LDREC(&pr[k * NT]) : dead;
-#if RA_LOOP_UNROLL == 2
-#pragma unroll 2
-#endif
                 while (leftW > 0) {
                     uint4 n[RA_ILP];
                     rach_u32x4 d[RA_ILP];
@@ -197,7 +182,7 @@ __global__ void __launch_bounds__(NT, MINB) ra_step_kernel(RaKernelArgs a) {
                     for (int k = 0; k < RA_ILP; ++k) {
                         RaPend land;
                         const bool lands = ra_phase1_mover_d<DUMP>(job, w, s, acc, T, i + k * NT, c[k], d[k], land);
-                        if (RA_DEFER && FIXED) {
+                        if (FIXED) {
                             /* a second re-transmitter in a lane that still holds one: the whole warp empties its registers
                              * (one pass of the list code for a dozen lanes instead of one pass per lane).  Only with the
                              * compile-time point view: with runtime parameters the three extra live registers cost more
@@ -211,17 +196,6 @@ __global__ void __launch_bounds__(NT, MINB) ra_step_kernel(RaKernelArgs a) {
                     i += RA_ILP * NT; pr += RA_ILP * NT; left -= RA_ILP * NT; leftW -= RA_ILP * NT;
                 }
                 ra_pend_flush(pt, w, s, T, pd);
-#else
-                uint4 c0 = i < nMov ? bT[i] : dead;
-                RaPend pd; pd.x = RA_INF32; pd.z = pd.w = 0;
-                while (i < nMov) {
-                    const unsigned ni = i + nt;
-                    const uint4 n0 = ni < nMov ? bT[ni] : dead;
-                    ra_phase1_mover<DUMP>(job, w, s, acc, T, i, c0, pd);
-                    c0 = n0; i = ni;
-                }
-                ra_pend_flush(pt, w, s, T, pd);
-#endif
                 const unsigned n1 = nMov + (unsigned)s.nArr + s.nM3;
                 for (i = nMov + tid; i < n1; i += nt) ra_phase1_item<DUMP>(job, w, s, acc, T, i);
                 __syncthreads();
@@ -647,10 +621,7 @@ static int ra_setup_device(ra_sim* sim, RaDev& d) {
                            : ra_step_entry(dump, shape, fixed, sim->opt.phaseTimers != 0);
     d.kern = kern;
     RA_CUDA(sim, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)d.smem));
-    /* the driver's default carveout heuristic was the best of {default, 50, 60, 75, 100 %} (within 0.6 %);
-     * RACH_CARVEOUT=<percent> overrides it for tuning */
-    if (const char* cv = getenv("RACH_CARVEOUT"))
-        RA_CUDA(sim, cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, atoi(cv)));
+    /* shared-memory carveout: the driver's default was the best of {default, 50, 60, 75, 100 %} (within 0.6 %) */
     int occ = 0;
     RA_CUDA(sim, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, d.nt, d.smem));
     if (occ < 1) { sim->err = "step kernel does not fit on an SM"; return RA_E_INVAL; }

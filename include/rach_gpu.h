@@ -101,10 +101,10 @@ typedef struct ra_stats {
 } ra_stats;
 
 /* Engine options (all zero = defaults).
- * Tuning / cross-check switches read from the environment at create / run time, never needed in normal use:
- *   RACH_BLOCK=big|small   force one of the two block shapes of the W step kernel (256 x 5 / 128 x 8 per SM)
- *   RACH_U0=serial         variant U0: the one-lane serial step in every ms instead of the warp step
- *   RACH_CARVEOUT=<pct>    preferred shared-memory carveout of the step kernel */
+ * Cross-check switches read from the environment at create / run time, never needed in normal use:
+ *   RACH_BLOCK=small|big|huge  force one of the three block shapes of the W/B step kernel (128 x 9 / 256 x 5 / 512 x 2 per SM)
+ *   RACH_FIXED=0               W/B: the runtime point view even when every point is in the reference's default family
+ *   RACH_U0=serial             variant U0: the one-lane serial step in every ms instead of the warp step */
 typedef struct ra_options {
     int repOffset;      /* tape replication id of local rep 0 (multi-process sharding)        */
     int dumpUEs;        /* 1 = keep the 16-int per-UE final record of every replication       */
