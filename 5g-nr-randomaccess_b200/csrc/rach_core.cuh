@@ -61,15 +61,6 @@ typedef unsigned long long ra_u64;
 #define RA_SCAP  512        /* singleton scans of one ms kept in shared memory (rest: global).  Shared memory is
                                kept small on purpose: at 5 resident blocks x 48 registers the spills live in L1 */
 #endif
-/* Optional shared-memory front of the per-ms work lists.  Measured on B200 with 1024 / 256 entries
- * (+20 KB per block): 12 % SLOWER than leaving the lists in the block's global workspace (L2-resident):
- * the smaller L1 costs more than the shorter small phases gain.  Default: all in global memory. */
-#ifndef RA_LCAP
-#define RA_LCAP  0          /* re-transmitters of one ms kept in shared memory (rest: global) */
-#endif
-#ifndef RA_UCAP
-#define RA_UCAP  0          /* uncertain movers of one ms kept in shared memory (rest: global) */
-#endif
 
 /* ---- atomics: CUDA on the device, plain read-modify-write in the host emulator ---------- */
 #ifdef __CUDA_ARCH__
@@ -133,7 +124,7 @@ struct RaPointDev {
     /* byte offsets of the block's tables in dynamic shared memory (ra_layout): a function of (R, P) only, kept
      * here so that a launch whose replications share one point reads them as kernel constants */
     unsigned oMinI, oCnt, oBcount, oM3count, oN, oL1, oNlList, oL1m, oL2, oBefore, oExtraFirst, oClsSize;
-    unsigned oHist, oSIdx, oSLand, oSLandMeta, oSUnc, smemBytes, oDead;
+    unsigned oHist, oSIdx, smemBytes, oDead;
     unsigned modSh;                        /* ra_mod_shift() of BI | P << 8 | A << 16 */
     /* rand() % backoffIndicator (W:514,540,685), rand() % nPreamble (W:478,502,701), subTime % accessTime (W:518) */
     RA_HDM unsigned modBI(unsigned x) const { return ra_mod(x, (unsigned)BI, magicBI, modSh & 0xFFu); }
@@ -141,17 +132,13 @@ struct RaPointDev {
     RA_HDM unsigned modA(unsigned x) const { return ra_mod(x, (unsigned)A, magicA, modSh >> 16); }
 };
 
-/* table layout for (R, P); 16-byte records first.  One definition for the runtime point (ra_layout) and for the
- * compile-time view below. */
+/* table layout for (R, P).  One definition for the runtime point (ra_layout) and for the compile-time view below. */
 struct RaLayout {
-    unsigned oSLand, oSUnc, oSLandMeta, oMinI, oCnt, oBcount, oDead, oM3count, oN, oL1, oNlList, oL1m, oL2, oBefore,
-             oExtraFirst, oClsSize, oHist, oSIdx, smemBytes;
+    unsigned oMinI, oCnt, oBcount, oDead, oM3count, oN, oL1, oNlList, oL1m, oL2, oBefore, oExtraFirst, oClsSize, oHist,
+             oSIdx, smemBytes;
 };
 #define RA_LAYOUT_BODY(R_, P_) \
     RaLayout l = {}; unsigned o = 0; const unsigned RP = (unsigned)(R_) * (unsigned)(P_), P4 = 4u * (unsigned)(P_); \
-    l.oSLand = o;      o += 16u * RA_LCAP; \
-    l.oSUnc = o;       o += 16u * RA_UCAP; \
-    l.oSLandMeta = o;  o += 4u * RA_LCAP; \
     l.oMinI = o;       o += 4u * RP; \
     l.oCnt = o;        o += 4u * RP; \
     l.oBcount = o;     o += 4u * (unsigned)(R_); \
@@ -183,8 +170,7 @@ template <int P_, int BI_, int A_, int Wn_, int R_>
 struct RaPointFixed : RaPointDev {
     static constexpr int P = P_, BI = BI_, A = A_, Wn = Wn_, R = R_;
     static constexpr RaLayout L = ra_layout_of(R_, P_);
-    static constexpr unsigned oSLand = L.oSLand, oSUnc = L.oSUnc, oSLandMeta = L.oSLandMeta, oMinI = L.oMinI, oCnt = L.oCnt,
-        oBcount = L.oBcount, oDead = L.oDead, oM3count = L.oM3count, oN = L.oN, oL1 = L.oL1, oNlList = L.oNlList, oL1m = L.oL1m, oL2 = L.oL2,
+    static constexpr unsigned oMinI = L.oMinI, oCnt = L.oCnt, oBcount = L.oBcount, oDead = L.oDead, oM3count = L.oM3count, oN = L.oN, oL1 = L.oL1, oNlList = L.oNlList, oL1m = L.oL1m, oL2 = L.oL2,
         oBefore = L.oBefore, oExtraFirst = L.oExtraFirst, oClsSize = L.oClsSize, oHist = L.oHist, oSIdx = L.oSIdx,
         smemBytes = L.smemBytes;
     RA_HDM unsigned modBI(unsigned x) const { return x % (unsigned)BI_; }
@@ -213,6 +199,31 @@ struct RaWork {
     unsigned* e1Meta;         /* [cap3] 1 = absorbed by a later scan                        */
     int cap, cap3;
 };
+
+/* the next 256-byte aligned table of `bytes` in a workspace at `base` (NULL: sizing only, no pointer) */
+static inline void* ra_carve_next(unsigned char* base, size_t& off, size_t bytes) {
+    void* p = base ? base + off : NULL;
+    off = (off + bytes + 255) / 256 * 256;
+    return p;
+}
+
+/* lays out one block's workspace at `base` for a ring of R move buckets and P preambles; returns its size in bytes */
+static inline size_t ra_work_carve(unsigned char* base, int cap, int cap3, int R, int P, RaWork* w) {
+    const size_t c = (size_t)cap, c3 = (size_t)cap3;
+    size_t off = 0;
+    w->bucket = (uint4*)ra_carve_next(base, off, sizeof(uint4) * c * (size_t)R);
+    w->msg3 = (uint4*)ra_carve_next(base, off, sizeof(uint4) * c3 * RA_M3RING);
+    w->landerRec = (uint4*)ra_carve_next(base, off, sizeof(uint4) * c);
+    w->landerMeta = (unsigned*)ra_carve_next(base, off, sizeof(unsigned) * c);
+    w->uncertain = (uint4*)ra_carve_next(base, off, sizeof(uint4) * c);
+    w->c3 = (uint4*)ra_carve_next(base, off, sizeof(uint4) * c);
+    w->singles = (unsigned*)ra_carve_next(base, off, sizeof(unsigned) * c);
+    w->e1Rec = (uint4*)ra_carve_next(base, off, sizeof(uint4) * c3);
+    w->e1Meta = (unsigned*)ra_carve_next(base, off, sizeof(unsigned) * c3);
+    w->minPos = (unsigned*)ra_carve_next(base, off, sizeof(unsigned) * (size_t)R * (size_t)P);
+    w->cap = cap; w->cap3 = cap3;
+    return off;
+}
 
 /* ---- per-CTA shared state ---------------------------------------------------------------- */
 struct RaShared {
@@ -296,7 +307,7 @@ static inline unsigned char* ra_smem() { return ra_emu_smem_base; }
 #endif
 #define RA_TAB_U(off)  (reinterpret_cast<unsigned*>(ra_smem() + (off)))
 #define RA_TAB_Q(off)  (reinterpret_cast<uint4*>(ra_smem() + (off)))
-struct RaTabsT { unsigned *minI, *cnt, *bcount, *dead, *m3count, *N, *l1, *nlList, *l1m, *l2, *before, *extraFirst, *clsSize, *hist, *sIdx, *sLandMeta; uint4 *sLand, *sUnc; };
+struct RaTabsT { unsigned *minI, *cnt, *bcount, *dead, *m3count, *N, *l1, *nlList, *l1m, *l2, *before, *extraFirst, *clsSize, *hist, *sIdx; };
 #define RA_T(name, O) (reinterpret_cast<decltype(RaTabsT::name)>(ra_smem() + pt.O))
 #define S_minI       RA_T(minI, oMinI)             /* [R*P] lowest UE index of the cohort                        */
 #define S_cnt        RA_T(cnt, oCnt)               /* [R*P] cohort size                                          */
@@ -313,13 +324,10 @@ struct RaTabsT { unsigned *minI, *cnt, *bcount, *dead, *m3count, *N, *l1, *nlLis
 #define S_clsSize    RA_T(clsSize, oClsSize)
 #define S_hist       RA_T(hist, oHist)             /* [RA_HBINS] singleton scans per index bin (grant selection) */
 #define S_sIdx       RA_T(sIdx, oSIdx)             /* [RA_SCAP]  first singleton indices of the ms                */
-#define S_sLand      RA_T(sLand, oSLand)           /* [RA_LCAP]  first re-transmitter records of the ms           */
-#define S_sLandMeta  RA_T(sLandMeta, oSLandMeta)   /* [RA_LCAP]                                                   */
-#define S_sUnc       RA_T(sUnc, oSUnc)             /* [RA_UCAP]  first uncertain movers of the ms                 */
 
 RA_HD void ra_layout(RaPointDev& pt) {
     const RaLayout l = ra_layout_of(pt.R, pt.P);
-    pt.oSLand = l.oSLand; pt.oSUnc = l.oSUnc; pt.oSLandMeta = l.oSLandMeta; pt.oMinI = l.oMinI; pt.oCnt = l.oCnt;
+    pt.oMinI = l.oMinI; pt.oCnt = l.oCnt;
     pt.oBcount = l.oBcount; pt.oDead = l.oDead; pt.oM3count = l.oM3count; pt.oN = l.oN; pt.oL1 = l.oL1; pt.oNlList = l.oNlList;
     pt.oL1m = l.oL1m; pt.oL2 = l.oL2; pt.oBefore = l.oBefore; pt.oExtraFirst = l.oExtraFirst; pt.oClsSize = l.oClsSize;
     pt.oHist = l.oHist; pt.oSIdx = l.oSIdx; pt.smemBytes = l.smemBytes;
@@ -330,22 +338,6 @@ RA_HD unsigned ra_first_scan(const PT& pt, unsigned p) {     /* s[p] of the head
     unsigned a = S_l1[p], b = S_l2[p];
     return a < b ? a : b;
 }
-
-/* per-ms work lists: the first entries live in shared memory (the small phases then never wait for
- * L2), the overflow in the block's global workspace */
-/* (x + 1 <= cap instead of x < cap: no "pointless comparison" diagnostics when a capacity is 0) */
-template <class PT>
-RA_HD uint4 ra_lrec_get(const PT& pt, const RaWork& w, unsigned l) { return l + 1 <= RA_LCAP ? S_sLand[l] : w.landerRec[l]; }
-template <class PT>
-RA_HD unsigned ra_lmeta_get(const PT& pt, const RaWork& w, unsigned l) { return l + 1 <= RA_LCAP ? S_sLandMeta[l] : w.landerMeta[l]; }
-template <class PT>
-RA_HD void ra_lmeta_set(const PT& pt, const RaWork& w, unsigned l, unsigned v) { if (l + 1 <= RA_LCAP) S_sLandMeta[l] = v; else w.landerMeta[l] = v; }
-template <class PT>
-RA_HD void ra_lmeta_add(const PT& pt, const RaWork& w, unsigned l, unsigned v) { if (l + 1 <= RA_LCAP) RA_AADD(&S_sLandMeta[l], v); else RA_AADD(&w.landerMeta[l], v); }
-template <class PT>
-RA_HD void ra_unc_set(const PT& pt, const RaWork& w, unsigned u, const uint4& e) { if (u + 1 <= RA_UCAP) S_sUnc[u] = e; else w.uncertain[u] = e; }
-template <class PT>
-RA_HD uint4 ra_unc_get(const PT& pt, const RaWork& w, unsigned u) { return u + 1 <= RA_UCAP ? S_sUnc[u] : w.uncertain[u]; }
 
 /* append a record to move bucket `m`; returns its position */
 template <class PT>
@@ -388,12 +380,10 @@ RA_HD void ra_msg3_push(const PT& pt, const RaWork& w, RaShared& s, int due, con
     w.msg3[(size_t)slot * w.cap3 + pos] = rec;
 }
 
-template <class PT>
-RA_HD void ra_lander_push(const PT& pt, const RaWork& w, RaShared& s, const uint4& rec, unsigned member) {
+RA_HD void ra_lander_push(const RaWork& w, RaShared& s, const uint4& rec, unsigned member) {
     unsigned l = RA_AADD(&s.nLanders, 1u);
     if (l >= (unsigned)w.cap) { s.overflow = 1; return; }
-    if (l + 1 <= RA_LCAP) { S_sLand[l] = rec; S_sLandMeta[l] = member; }
-    else { w.landerRec[l] = rec; w.landerMeta[l] = member; }
+    w.landerRec[l] = rec; w.landerMeta[l] = member;
 }
 
 /* ---- dump helpers (DUMP builds only) ------------------------------------------------------ */
@@ -506,14 +496,15 @@ RA_HD void ra_pend_flush(const PT& pt, const RaWork& w, RaShared& s, int T, RaPe
     if (pd.x == RA_INF32) return;
     const unsigned idx = pd.x & 0x7FFFFFFFu;
     RA_AMIN(&S_l2[pd.w & 0xFFu], idx);
-    ra_lander_push(pt, w, s, make_uint4(idx, (unsigned)T, pd.z, pd.w), pd.x >> 31);
+    ra_lander_push(w, s, make_uint4(idx, (unsigned)T, pd.z, pd.w), pd.x >> 31);
     pd.x = RA_INF32;
 }
 
 template <bool DUMP, class PT>
 RA_HD bool ra_phase1_mover_d(const RaJobT<PT>& job, const RaWork& w, RaShared& s, RaAcc& acc, int T, unsigned item, const uint4& rec, const rach_u32x4& d, RaPend& land);
 
-/* one mover, its re-transmission (if any) parked in `pd` (the caller flushes it before the phase ends) */
+/* one mover, its re-transmission (if any) parked in `pd` (the caller flushes it before the phase ends): the mover loop of
+ * the kernel one record at a time (used by the host emulation) */
 template <bool DUMP, class PT>
 RA_HD void ra_phase1_mover(const RaJobT<PT>& job, const RaWork& w, RaShared& s, RaAcc& acc, int T, unsigned item, const uint4& rec, RaPend& pd) {
     if (rec.x == RA_DEAD) return;
@@ -524,8 +515,9 @@ RA_HD void ra_phase1_mover(const RaJobT<PT>& job, const RaWork& w, RaShared& s, 
     }
 }
 
-/* the draws of (UE, T) are passed in so that the kernel can run two Philox chains side by side.  Returns true if the
- * UE re-transmits in this ms: its new record is then in `land` and has NOT been put on the work list. */
+/* one mover (work item `item` < nMov); the draws of (UE, T) are passed in so that the kernel can run two Philox chains
+ * side by side.  Returns true if the UE re-transmits in this ms: its new record is then in `land` and has NOT been put
+ * on the work list. */
 template <bool DUMP, class PT>
 RA_HD bool ra_phase1_mover_d(const RaJobT<PT>& job, const RaWork& w, RaShared& s, RaAcc& acc, int T, unsigned item, const uint4& rec, const rach_u32x4& d, RaPend& land) {
     const PT& pt = *job.pt;
@@ -559,7 +551,7 @@ RA_HD bool ra_phase1_mover_d(const RaJobT<PT>& job, const RaWork& w, RaShared& s
     land.z = z; land.w = nw;                               /* (assigned on every path: the values stay in registers) */
     if (uncertain) {
         unsigned u = RA_AADD(&s.nUnc, 1u);
-        ra_unc_set(pt, w, u, make_uint4(item, idx, p0 | (limit ? 0x80000000u : 0u), 0));
+        w.uncertain[u] = make_uint4(item, idx, p0 | (limit ? 0x80000000u : 0u), 0);
         if (limit) {
             if (X == T) { unsigned c = RA_AADD(&s.nC3, 1u); w.c3[c] = make_uint4(idx, p0, pnew, 0); }
             return false;
@@ -635,16 +627,9 @@ RA_HD int ra_msg3_item(const RaJobT<PT>& job, const RaWork& w, RaShared& s, RaAc
     return 0;
 }
 
+/* the events after the movers: item >= nMov */
 template <bool DUMP, class PT>
 RA_HD void ra_phase1_item(const RaJobT<PT>& job, const RaWork& w, RaShared& s, RaAcc& acc, int T, unsigned item) {
-    const PT& pt = *job.pt;
-    const unsigned Rm = (unsigned)(pt.R - 1);
-    if (item < s.nMov) {
-        RaPend pd; pd.x = RA_INF32; pd.z = pd.w = 0;
-        ra_phase1_mover<DUMP>(job, w, s, acc, T, item, w.bucket[(size_t)((unsigned)T & Rm) * w.cap + item], pd);
-        ra_pend_flush(pt, w, s, T, pd);
-        return;
-    }
     item -= s.nMov;
     if (item < (unsigned)s.nArr) { ra_arrival_item<DUMP>(job, w, s, T, (unsigned)s.acOld + item); return; }
     item -= (unsigned)s.nArr;
@@ -677,7 +662,7 @@ RA_HD void ra_phase2_serial(const PT& pt, const RaWork& w, RaShared& s) {
 template <bool DUMP, class PT>
 RA_HD void ra_phase3_item(const RaJobT<PT>& job, const RaWork& w, RaShared& s, int T, unsigned u) {
     const PT& pt = *job.pt;
-    const uint4 e = ra_unc_get(pt, w, u);
+    const uint4 e = w.uncertain[u];
     const unsigned idx = e.y, p0 = e.z & 0xFFu;
     const unsigned sp = ra_first_scan(pt, p0);
     if (idx < sp) RA_AADD(&S_before[p0], 1u);              /* left the class before its first scan */
@@ -691,7 +676,7 @@ RA_HD void ra_phase3_item(const RaJobT<PT>& job, const RaWork& w, RaShared& s, i
     int X = ra_align_pt(pt, base + tmp);
     uint4 nr = make_uint4(idx, (unsigned)X, ra_z((unsigned)T, ra_rec_fail(rec) + 1), ra_w3(pnew, 0, 1, 0));
     if (DUMP) job.dump[(size_t)idx * RA_DUMP_W + 3] = T + 1;
-    if (X == T) ra_lander_push(pt, w, s, nr, pnew == p0 ? 1u : 0u);   /* S_l2 already holds it (phase 2) */
+    if (X == T) ra_lander_push(w, s, nr, pnew == p0 ? 1u : 0u);   /* S_l2 already holds it (phase 2) */
     else ra_schedule(pt, w, s, nr);                         /* X > T always: base >= T */
 }
 
@@ -707,13 +692,13 @@ RA_HD void ra_phase3b_item(const PT& pt, const RaWork& w, RaShared& s, unsigned 
     unsigned sq = ra_first_scan(pt, q);
     if (sq != RA_INF32 && sq > k && sq == S_l1[q]) { bestIdx = sq; bestRef = 0x80000000u | q; }
     for (unsigned l = 0; l < s.nLanders; ++l) {
-        const uint4 lr = ra_lrec_get(pt, w, l);
+        const uint4 lr = w.landerRec[l];
         if (ra_rec_p(lr) == q && lr.x > k && lr.x < bestIdx) { bestIdx = lr.x; bestRef = l; }
     }
     if (bestIdx == RA_INF32) return;
     w.e1Meta[e] = 1;
     if (bestRef & 0x80000000u) RA_AADD(&S_extraFirst[q], 1u);
-    else ra_lmeta_add(pt, w, bestRef, 256u);
+    else RA_AADD(&w.landerMeta[bestRef], 256u);
 }
 
 /* =========================================================================================
@@ -721,6 +706,10 @@ RA_HD void ra_phase3b_item(const PT& pt, const RaWork& w, RaShared& s, unsigned 
  *   class items  [0, P):        first scan by the natural leader (a visible non-mover)
  *   lander items [P, P+nLanders): scan by a UE that re-transmits in this ms
  * ========================================================================================= */
+/* singleton j of the ms: the first RA_SCAP in shared memory, all of them in the workspace */
+template <class PT>
+RA_HD unsigned ra_single(const PT& pt, const RaWork& w, unsigned j) { return j < RA_SCAP ? S_sIdx[j] : w.singles[j]; }
+
 template <class PT>
 RA_HD void ra_single_push(const PT& pt, const RaWork& w, RaShared& s, unsigned idx) {
     unsigned k = RA_AADD(&s.nSingles, 1u);
@@ -751,8 +740,8 @@ RA_HD void ra_phase4_item(const PT& pt, const RaWork& w, RaShared& s, RaAcc& acc
     }
     const unsigned l = item - (unsigned)pt.P;
     if (l >= s.nLanders) return;
-    const uint4 r = ra_lrec_get(pt, w, l);
-    const unsigned q = ra_rec_p(r), meta = ra_lmeta_get(pt, w, l);
+    const uint4 r = w.landerRec[l];
+    const unsigned q = ra_rec_p(r), meta = w.landerMeta[l];
     unsigned size;
     if (r.x == ra_first_scan(pt, q)) size = S_N[q] - S_before[q] + ((meta & 1u) ? 0u : 1u) + (meta >> 8);
     else size = 1u + (meta >> 8);
@@ -760,15 +749,19 @@ RA_HD void ra_phase4_item(const PT& pt, const RaWork& w, RaShared& s, RaAcc& acc
     if (size == 1) {
         ra_single_push(pt, w, s, r.x);
     } else {
-        ra_lmeta_set(pt, w, l, meta | 2u);                   /* collided */
+        w.landerMeta[l] = meta | 2u;                        /* collided */
     }
 }
 
 /* =========================================================================================
- * Phase 5 (one thread / warp) -- UL grants: the first G-1-grantCheck singleton scans in UE
- * index order are granted (strict '<' after the increment, W:639-641).
+ * Phase 5 (one warp, vector form of rach_warp.cuh) -- UL grants: the first G-1-grantCheck
+ * singleton scans in UE index order are granted (strict '<' after the increment, W:639-641).
  * tau = highest granted index (RA_INF32: all, 0 with nobody granted handled by flag).
+ * Histogram over index bins (filled by phase 4) -> the bin holding the K-th smallest -> exact
+ * rank inside that bin.
  * ========================================================================================= */
+/* the same threshold by one thread, straight from the definition: the reference formulation the host emulation checks
+ * ra_phase5_warp against */
 template <class PT>
 RA_HD void ra_phase5_serial(const PT& pt, const RaWork& w, RaShared& s) {
     const unsigned n = s.nSingles;
@@ -791,11 +784,8 @@ RA_HD void ra_phase5_serial(const PT& pt, const RaWork& w, RaShared& s) {
     s.grantCheck += (int)n;
 }
 
-#ifdef __CUDACC__
-/* the same threshold computed by one warp: histogram over index bins (filled by phase 4) ->
- * the bin holding the K-th smallest -> exact rank inside that bin */
 template <class PT>
-__device__ __forceinline__ void ra_phase5_warp(const PT& pt, const RaWork& w, RaShared& s, int lane) {
+RW_FN void ra_phase5_warp(const PT& pt, const RaWork& w, RaShared& s) {
     const unsigned n = s.nSingles;
     long long K = (long long)pt.G - 1 - s.grantCheck;
     if (K < 0) K = 0;
@@ -806,47 +796,55 @@ __device__ __forceinline__ void ra_phase5_warp(const PT& pt, const RaWork& w, Ra
             /* at most one singleton per lane (the normal case away from the overload peak, where the singletons of a ms are
              * the UEs of one arrival step -- consecutive indices, all in ONE histogram bin, so the bin walk below would
              * take K full passes): rank by counting, the K-th smallest is the lane whose rank is K - 1 (indices are distinct) */
-            const unsigned v = (unsigned)lane < n ? S_sIdx[lane] : RA_INF32;       /* n <= 32 <= RA_SCAP */
-            unsigned rank = 0;
-            for (unsigned i = 0; i < n; ++i) rank += __shfl_sync(0xFFFFFFFFu, v, (int)i) < v ? 1u : 0u;
-            const unsigned hit = __ballot_sync(0xFFFFFFFFu, (unsigned)lane < n && rank == (unsigned)K - 1u);
-            tau = __shfl_sync(0xFFFFFFFFu, v, __ffs((int)hit) - 1);
+            unsigned v[RW_LANES];
+            int hit[RW_LANES];
+            RW_EACH(l) v[l] = (unsigned)lane < n ? ra_single(pt, w, (unsigned)lane) : RA_INF32;
+            RW_EACH(l) {
+                unsigned rank = 0;
+                for (unsigned i = 0; i < n; ++i) rank += RW_SHFL(v, (int)i) < v[l] ? 1u : 0u;
+                hit[l] = (unsigned)lane < n && rank == (unsigned)K - 1u;
+            }
+            tau = RW_SHFL(v, RW_FFS(RW_BALLOT(hit)) - 1);
         }
         else {
             const unsigned k = (unsigned)K;
             const int per = RA_HBINS / 32;
-            unsigned sum = 0;
-            for (int b = 0; b < per; ++b) sum += S_hist[lane * per + b];
-            unsigned incl = sum;
-            for (int o = 1; o < 32; o <<= 1) { unsigned v = __shfl_up_sync(0xFFFFFFFFu, incl, o); if (lane >= o) incl += v; }
-            const int L = __ffs(__ballot_sync(0xFFFFFFFFu, incl >= k)) - 1;
-            unsigned bstar = 0, before = 0;
-            if (lane == L) {
-                unsigned c = incl - sum;
-                for (int b = 0; b < per; ++b) {
-                    unsigned h = S_hist[lane * per + b];
-                    if (c + h >= k) { bstar = (unsigned)(lane * per + b); before = c; break; }
-                    c += h;
+            unsigned sum[RW_LANES], incl[RW_LANES], bstar[RW_LANES], before[RW_LANES];
+            int ge[RW_LANES];
+            RW_EACH(l) { sum[l] = 0; for (int b = 0; b < per; ++b) sum[l] += S_hist[lane * per + b]; }
+            rw_scan_u32(sum, incl);
+            RW_EACH(l) ge[l] = incl[l] >= k;
+            const int L = RW_FFS(RW_BALLOT(ge)) - 1;
+            RW_EACH(l) {
+                bstar[l] = 0; before[l] = 0;
+                if (lane == L) {
+                    unsigned c = incl[l] - sum[l];
+                    for (int b = 0; b < per; ++b) {
+                        const unsigned h = S_hist[lane * per + b];
+                        if (c + h >= k) { bstar[l] = (unsigned)(lane * per + b); before[l] = c; break; }
+                        c += h;
+                    }
                 }
             }
-            bstar = __shfl_sync(0xFFFFFFFFu, bstar, L); before = __shfl_sync(0xFFFFFFFFu, before, L);
-            const unsigned kk = k - before;                 /* 1-based rank inside bin bstar */
+            const unsigned bin = RW_SHFL(bstar, L);
+            const unsigned kk = k - RW_SHFL(before, L);     /* 1-based rank inside bin `bin` */
             unsigned prev = 0; bool first = true;
             for (unsigned r = 0; r < kk; ++r) {
-                unsigned best = RA_INF32;
-                for (unsigned j = lane; j < n; j += 32) {
-                    unsigned v = j < RA_SCAP ? S_sIdx[j] : w.singles[j];
-                    if ((v >> pt.hshift) == bstar && (first || v > prev) && v < best) best = v;
+                unsigned best[RW_LANES];
+                RW_EACH(l) {
+                    best[l] = RA_INF32;
+                    for (unsigned j = lane; j < n; j += 32) {
+                        const unsigned x = ra_single(pt, w, j);
+                        if ((x >> pt.hshift) == bin && (first || x > prev) && x < best[l]) best[l] = x;
+                    }
                 }
-                for (int o = 16; o; o >>= 1) { unsigned v = __shfl_xor_sync(0xFFFFFFFFu, best, o); best = v < best ? v : best; }
-                prev = best; first = false;
+                prev = rw_min_u32(best); first = false;
             }
             tau = prev;
         }
     }
-    if (lane == 0) { s.tau = tau; s.noGrant = noGrant; s.grantCheck += (int)n; }
+    RW_EACH(l) if (lane == 0) { s.tau = tau; s.noGrant = noGrant; s.grantCheck += (int)n; }
 }
-#endif
 
 RA_HD bool ra_granted(const RaShared& s, unsigned idx) { return !s.noGrant && idx <= s.tau; }
 
@@ -907,8 +905,8 @@ RA_HD void ra_phase6_item(const RaJobT<PT>& job, const RaWork& w, RaShared& s, i
     }
     item -= (unsigned)pt.P;
     if (item < s.nLanders) {
-        uint4 r = ra_lrec_get(pt, w, item);
-        const unsigned meta = ra_lmeta_get(pt, w, item);
+        uint4 r = w.landerRec[item];
+        const unsigned meta = w.landerMeta[item];
         if (!(meta & 2u) && ra_granted(s, r.x)) {
             if (DUMP) { int* row = job.dump + (size_t)r.x * RA_DUMP_W; row[8] = 0; row[9] = (int)ra_rec_mrc(r); }
             r.y = (unsigned)(T + 11);
@@ -949,7 +947,7 @@ template <class PT>
 RA_HD void ra_hist_clear(const PT& pt, const RaWork& w, RaShared& s, int tid, int nt) {
     const unsigned n = s.nSingles;
     if (n > RA_HBINS / 2) { for (int i = tid; i < RA_HBINS; i += nt) S_hist[i] = 0; }
-    else for (unsigned j = tid; j < n; j += nt) S_hist[(j < RA_SCAP ? S_sIdx[j] : w.singles[j]) >> pt.hshift] = 0;
+    else for (unsigned j = tid; j < n; j += nt) S_hist[ra_single(pt, w, j) >> pt.hshift] = 0;
 }
 
 /* =========================================================================================
@@ -969,18 +967,6 @@ RA_HD void ra_hist_clear(const PT& pt, const RaWork& w, RaShared& s, int tid, in
  *            path from the class view (ra_phase0_classes) and phase 2
  *         3  complete except for a granted UE whose position hint was stale: run ra_phase6b
  * ========================================================================================= */
-RW_FN unsigned rw_min_u32(const unsigned* a) {
-#ifdef __CUDA_ARCH__
-    unsigned v = a[0];
-    for (int o = 16; o > 0; o >>= 1) { const unsigned t = __shfl_xor_sync(0xFFFFFFFFu, v, o); v = t < v ? t : v; }
-    return v;
-#else
-    unsigned v = a[0];
-    for (int i = 1; i < 32; ++i) v = a[i] < v ? a[i] : v;
-    return v;
-#endif
-}
-
 /* the control block of the replication as warp-uniform registers: warp 0 keeps it there while it runs light ms back to
  * back (every lane computes the same updates) and writes it back to shared memory when the block takes over */
 struct RaCtl { int grantCheck, activeCheck, nextAc, nextArrMs, occ; unsigned nM3sum; };

@@ -70,6 +70,18 @@ struct RaWorkN {
     int cap, cap3;
 };
 
+/* lays out one block's workspace at `base` for a ring of R buckets; returns its size in bytes (ra_work_carve) */
+static inline size_t rn_work_carve(unsigned char* base, int cap, int cap3, int R, RaWorkN* w) {
+    const size_t c = (size_t)cap, c3 = (size_t)cap3;
+    size_t off = 0;
+    w->bucket = (uint4*)ra_carve_next(base, off, sizeof(uint4) * c * (size_t)R);
+    w->msg3 = (uint4*)ra_carve_next(base, off, sizeof(uint4) * c3 * RA_M3RING);
+    w->zombie = (uint4*)ra_carve_next(base, off, sizeof(uint4) * c);
+    w->gain = (double*)ra_carve_next(base, off, sizeof(double) * c);
+    w->cap = cap; w->cap3 = cap3;
+    return off;
+}
+
 struct RaSharedN {
     unsigned* cnt;       /* [6*P] transmitters per (sector, preamble)                         */
     unsigned* who;       /* [6*P] bucket position of the first one                            */
@@ -85,6 +97,24 @@ struct RaSharedN {
     unsigned nSuccess, nZombie, nDropped, pad;
     ra_u64 txSum, delaySum;
 };
+
+/* the block's tables in dynamic shared memory (the kernel's; the host emulation carves a host buffer the same way) */
+RA_HD void rn_carve(RaSharedN& s, unsigned char* base, int R, int P) {
+    const size_t c = (size_t)RA_NSECT * P;
+    s.sLg = reinterpret_cast<double*>(base);     base += sizeof(double) * c;
+    s.sGain = reinterpret_cast<double*>(base);   base += sizeof(double) * c;
+    s.cnt = reinterpret_cast<unsigned*>(base);   base += sizeof(unsigned) * c;
+    s.who = reinterpret_cast<unsigned*>(base);   base += sizeof(unsigned) * c;
+    s.grant = reinterpret_cast<unsigned*>(base); base += sizeof(unsigned) * c;
+    s.sPos = reinterpret_cast<unsigned*>(base);  base += sizeof(unsigned) * c;
+    s.sIdx = reinterpret_cast<int*>(base);       base += sizeof(int) * c;
+    s.ord = reinterpret_cast<unsigned*>(base);   base += sizeof(unsigned) * c;
+    s.bcount = reinterpret_cast<unsigned*>(base); base += sizeof(unsigned) * (size_t)R;
+    s.m3count = reinterpret_cast<unsigned*>(base);
+}
+RA_HD size_t rn_smem_bytes(int R, int P) {
+    return (size_t)RA_NSECT * P * (2 * sizeof(double) + 6 * sizeof(unsigned)) + sizeof(unsigned) * ((size_t)R + RA_M3RING);
+}
 
 /* UE draw stream of one (ue, ms): draw k is word k&3 of block k>>2 */
 struct RaStream {

@@ -37,6 +37,12 @@ struct RU_ALIGN RuUE {   /* 64 bytes; the first 16 are all a collision scan read
     int raFailed, nowBackoff, pad0, pad1;   /* pad0: next node of a phantom chain */
 };
 
+/* RuUE entries of one replication's global workspace: live-list overflow [cap], phantom store [cap], phantom calendar
+ * heads [maxR ints] */
+RA_HD size_t ru_work_elems(int cap, int maxR) {
+    return 2 * (size_t)cap + ((size_t)maxR * sizeof(int) + sizeof(RuUE) - 1) / sizeof(RuUE);
+}
+
 struct RuStats { int simTime, nSuccess; long long txSum, delaySum, collisionPreambles, totalPreambleTxop, dropped; int overflow; };
 
 /* dump row: timer active txTime preamble preambleChange rarWindow maxRarCounter preambleTxCounter

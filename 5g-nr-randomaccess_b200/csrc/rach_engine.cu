@@ -229,7 +229,7 @@ __global__ void __launch_bounds__(NT, MINB) ra_step_kernel(RaKernelArgs a) {
                 if (ra_phase5_trivial(pt, s)) {                    /* every scan answered: no threshold, no barrier */
                     if (tid == 0) s.gcAdd = (int)s.nSingles;
                 } else {
-                    if (tid < 32) ra_phase5_warp(pt, w, s, tid);
+                    if (tid < 32) ra_phase5_warp(pt, w, s);
                     __syncthreads();
                     RA_TICK(6);
                 }
@@ -283,23 +283,6 @@ __global__ void __launch_bounds__(NT, MINB) ra_step_kernel(RaKernelArgs a) {
 /* ------------------------------------------------------------------------------------------
  * Variant N (NOMA.c): one block per replication, phases of rach_core_n.cuh.
  * ------------------------------------------------------------------------------------------ */
-__device__ __forceinline__ void rn_carve(RaSharedN& s, unsigned char* base, int R, int P) {
-    const size_t c = (size_t)RA_NSECT * P;
-    s.sLg = reinterpret_cast<double*>(base);     base += sizeof(double) * c;
-    s.sGain = reinterpret_cast<double*>(base);   base += sizeof(double) * c;
-    s.cnt = reinterpret_cast<unsigned*>(base);   base += sizeof(unsigned) * c;
-    s.who = reinterpret_cast<unsigned*>(base);   base += sizeof(unsigned) * c;
-    s.grant = reinterpret_cast<unsigned*>(base); base += sizeof(unsigned) * c;
-    s.sPos = reinterpret_cast<unsigned*>(base);  base += sizeof(unsigned) * c;
-    s.sIdx = reinterpret_cast<int*>(base);       base += sizeof(int) * c;
-    s.ord = reinterpret_cast<unsigned*>(base);   base += sizeof(unsigned) * c;
-    s.bcount = reinterpret_cast<unsigned*>(base); base += sizeof(unsigned) * (size_t)R;
-    s.m3count = reinterpret_cast<unsigned*>(base);
-}
-static size_t rn_smem_bytes(int R, int P) {
-    return (size_t)RA_NSECT * P * (2 * sizeof(double) + 6 * sizeof(unsigned)) + sizeof(unsigned) * ((size_t)R + RA_M3RING);
-}
-
 template <bool DUMP>
 __global__ void __launch_bounds__(RA_NT_N, RA_MINB_N) ra_step_kernel_n(RaKernelArgs a) {     /* fp64 activation math: 64 registers, no spills */
     extern __shared__ __align__(16) unsigned char ra_dyn_smem[];
@@ -394,9 +377,7 @@ template <bool DUMP>
 __global__ void __launch_bounds__(32) ra_u0_kernel(RaKernelArgs a, int cap, int headsInSmem, int lanesOn) {
     extern __shared__ __align__(16) unsigned char ru_dyn_smem[];
     const int lane = threadIdx.x;
-    /* per block: live-list overflow [cap], phantom store [cap], phantom calendar heads [maxR ints] */
-    const size_t perBlock = 2 * (size_t)cap + ((size_t)a.maxR * sizeof(int) + sizeof(RuUE) - 1) / sizeof(RuUE);
-    RuUE* live = a.liveBase + (size_t)blockIdx.x * perBlock;
+    RuUE* live = a.liveBase + (size_t)blockIdx.x * ru_work_elems(cap, a.maxR);
     RuUE* ph = live + cap;
     int* phHead = reinterpret_cast<int*>(ph + cap);
     RuUE* win = reinterpret_cast<RuUE*>(ru_dyn_smem);
@@ -525,8 +506,6 @@ static void ra_free_dev(RaDev& d) {
     if (d.hDone) cudaFreeHost(d.hDone);
 }
 
-static size_t ra_align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
-
 static int ra_setup_device(ra_sim* sim, RaDev& d) {
     RA_CUDA(sim, cudaSetDevice(d.id));
     cudaDeviceProp prop;
@@ -572,7 +551,7 @@ static int ra_setup_device(ra_sim* sim, RaDev& d) {
         /* one warp (block) per replication; global live-list overflow + phantom store of cap UEs (64 B each) per block */
         size_t freeB = 0, totalB = 0;
         RA_CUDA(sim, cudaMemGetInfo(&freeB, &totalB));
-        const size_t perThread = sizeof(RuUE) * (2 * (size_t)sim->cap + ((size_t)sim->maxR * sizeof(int) + sizeof(RuUE) - 1) / sizeof(RuUE));
+        const size_t perThread = sizeof(RuUE) * ru_work_elems(sim->cap, sim->maxR);
         long long threads = std::min<long long>(nJobs, (long long)((double)freeB * 0.85 / (double)perThread));
         threads = std::min<long long>(threads, (long long)prop.multiProcessorCount * 32);   /* resident blocks */
         if (threads < 1) { sim->err = "not enough device memory for one U0 live list"; return RA_E_NOMEM; }
@@ -631,19 +610,9 @@ static int ra_setup_device(ra_sim* sim, RaDev& d) {
         if (e != cudaSuccess) { sim->err = "gain dump buffer does not fit on the device"; return RA_E_NOMEM; }
     }
 
-    const size_t cap = (size_t)sim->cap, cap3 = (size_t)sim->cap3;
-    size_t off = 0;
-    const size_t oBucket = off;    off = ra_align_up(off + sizeof(uint4) * cap * sim->maxR, 256);
-    const size_t oMsg3 = off;      off = ra_align_up(off + sizeof(uint4) * cap3 * RA_M3RING, 256);
-    const size_t oLander = off;    off = ra_align_up(off + sizeof(uint4) * cap, 256);               /* N: zombies */
-    const size_t oLMeta = off;     off = ra_align_up(off + (isN ? sizeof(double) : sizeof(unsigned)) * cap, 256);   /* N: gains */
-    const size_t oUnc = off;       if (!isN) off = ra_align_up(off + sizeof(uint4) * cap, 256);
-    const size_t oC3 = off;        if (!isN) off = ra_align_up(off + sizeof(uint4) * cap, 256);
-    const size_t oSingles = off;   if (!isN) off = ra_align_up(off + sizeof(unsigned) * cap, 256);
-    const size_t oE1 = off;        if (!isN) off = ra_align_up(off + sizeof(uint4) * cap3, 256);
-    const size_t oE1Meta = off;    if (!isN) off = ra_align_up(off + sizeof(unsigned) * cap3, 256);
-    const size_t oMinPos = off;    if (!isN) off = ra_align_up(off + sizeof(unsigned) * (size_t)sim->maxR * sim->maxP, 256);
-    const size_t perBlock = off;
+    RaWork sizeW; RaWorkN sizeN;
+    const size_t perBlock = isN ? rn_work_carve(nullptr, sim->cap, sim->cap3, sim->maxR, &sizeN)
+                                : ra_work_carve(nullptr, sim->cap, sim->cap3, sim->maxR, sim->maxP, &sizeW);
 
     size_t freeB = 0, totalB = 0;
     RA_CUDA(sim, cudaMemGetInfo(&freeB, &totalB));
@@ -658,27 +627,13 @@ static int ra_setup_device(ra_sim* sim, RaDev& d) {
     }
     if (isN) {
         std::vector<RaWorkN> worksN(grid);
-        for (int b = 0; b < grid; ++b) {
-            unsigned char* base = d.dWorkspace + perBlock * (size_t)b;
-            RaWorkN& w = worksN[b];
-            w.bucket = (uint4*)(base + oBucket); w.msg3 = (uint4*)(base + oMsg3);
-            w.zombie = (uint4*)(base + oLander); w.gain = (double*)(base + oLMeta);
-            w.cap = sim->cap; w.cap3 = sim->cap3;
-        }
+        for (int b = 0; b < grid; ++b) rn_work_carve(d.dWorkspace + perBlock * (size_t)b, sim->cap, sim->cap3, sim->maxR, &worksN[b]);
         RA_CUDA(sim, cudaMalloc(&d.dWorksN, sizeof(RaWorkN) * grid));
         RA_CUDA(sim, cudaMemcpy(d.dWorksN, worksN.data(), sizeof(RaWorkN) * grid, cudaMemcpyHostToDevice));
         return RA_OK;
     }
     std::vector<RaWork> works(grid);
-    for (int b = 0; b < grid; ++b) {
-        unsigned char* base = d.dWorkspace + perBlock * (size_t)b;
-        RaWork& w = works[b];
-        w.bucket = (uint4*)(base + oBucket); w.msg3 = (uint4*)(base + oMsg3);
-        w.landerRec = (uint4*)(base + oLander); w.landerMeta = (unsigned*)(base + oLMeta);
-        w.uncertain = (uint4*)(base + oUnc); w.c3 = (uint4*)(base + oC3);
-        w.singles = (unsigned*)(base + oSingles); w.e1Rec = (uint4*)(base + oE1);
-        w.e1Meta = (unsigned*)(base + oE1Meta); w.minPos = (unsigned*)(base + oMinPos); w.cap = sim->cap; w.cap3 = sim->cap3;
-    }
+    for (int b = 0; b < grid; ++b) ra_work_carve(d.dWorkspace + perBlock * (size_t)b, sim->cap, sim->cap3, sim->maxR, sim->maxP, &works[b]);
     RA_CUDA(sim, cudaMalloc(&d.dWorks, sizeof(RaWork) * grid));
     RA_CUDA(sim, cudaMemcpy(d.dWorks, works.data(), sizeof(RaWork) * grid, cudaMemcpyHostToDevice));
     return RA_OK;
@@ -711,13 +666,8 @@ extern "C" ra_sim* ra_sim_create_ex(const ra_params* points, int nPoints, int re
         const ra_params& p = points[i];
         if (i == 0) sim->variant = p.variant;
         else if (p.variant != sim->variant) { g_createErr = "all points of one ra_sim must share the variant"; delete sim; return nullptr; }
-        RaPointDev pt; memset(&pt, 0, sizeof pt);
-        pt.nUE = p.nUE; pt.P = p.nPreamble; pt.BI = p.backoffIndicator; pt.G = p.nGrantUL;
-        pt.Wn = p.maxRarWindow; pt.M = p.maxMsg2TxCount; pt.A = p.accessTime;
-        pt.maxTime = ra_horizon_ms(&p); pt.geometry = p.geometry ? 1 : 0; pt.R = ra_host_ring(&p);
-        pt.nOcc = (pt.maxTime + pt.A - 1) / pt.A; pt.seed = p.seed; pt.arrCum = nullptr; pt.cellRadius = p.cellRadius;
-        ra_host_fill_point(&pt);
-        if (p.variant == RA_VARIANT_U0) ra_host_point_u0(&p, &pt);
+        RaPointDev pt;
+        ra_host_point(&p, &pt);
         sim->hostPoints.push_back(pt);
         sim->arrCum.emplace_back(pt.nOcc);
         ra_host_arrcum(&p, sim->arrCum.back().data(), pt.nOcc);
@@ -731,8 +681,7 @@ extern "C" ra_sim* ra_sim_create_ex(const ra_params* points, int nPoints, int re
         }
         sim->maxP = std::max(sim->maxP, pt.P); sim->maxR = std::max(sim->maxR, pt.R);
         sim->cap = std::max(sim->cap, pt.nUE);
-        long long g2 = (p.variant == RA_VARIANT_N ? 24LL : 2LL) * std::min<long long>(pt.G, (long long)pt.nUE + 1) + 4;
-        sim->cap3 = std::max<long long>(sim->cap3, g2);
+        sim->cap3 = std::max(sim->cap3, ra_host_cap3(p.variant, &pt));
         sim->dumpStride = std::max(sim->dumpStride, (size_t)pt.nUE * RA_DUMP_W);
     }
     /* the engines index a block's move calendar with 32 bits (ring x capacity records of 16 bytes: 64 GB) */

@@ -173,7 +173,7 @@ void ra_host_fill_point(RaPointDev* pt) {
     ra_layout(*pt);
 }
 
-/* variant U0: RaPointDev.G carries nAccessUE = ceil(n*5/60000), at least 1 (U0:60-64) */
+/* variant U0: RaPointDev.G carries nAccessUE = ceil(n*5/60000), at least 1 (U0:60-64); no arrival schedule (nOcc 0) */
 void ra_host_point_u0(const ra_params* p, RaPointDev* pt) {
     memset(pt, 0, sizeof *pt);
     pt->nUE = p->nUE; pt->P = p->nPreamble; pt->BI = p->backoffIndicator; pt->A = 5;
@@ -184,6 +184,21 @@ void ra_host_point_u0(const ra_params* p, RaPointDev* pt) {
     if (nAccessUE == 0) nAccessUE = 1;
     pt->G = nAccessUE;
     ra_host_fill_point(pt);
+}
+
+void ra_host_point(const ra_params* p, RaPointDev* pt) {
+    if (p->variant == RA_VARIANT_U0) { ra_host_point_u0(p, pt); return; }
+    memset(pt, 0, sizeof *pt);
+    pt->nUE = p->nUE; pt->P = p->nPreamble; pt->BI = p->backoffIndicator; pt->G = p->nGrantUL;
+    pt->Wn = p->maxRarWindow; pt->M = p->maxMsg2TxCount; pt->A = p->accessTime;
+    pt->maxTime = ra_horizon_ms(p); pt->geometry = p->geometry ? 1 : 0; pt->R = ra_host_ring(p);
+    pt->nOcc = (pt->maxTime + pt->A - 1) / pt->A; pt->seed = p->seed; pt->cellRadius = p->cellRadius;
+    ra_host_fill_point(pt);
+}
+
+int ra_host_cap3(int variant, const RaPointDev* pt) {
+    const long long g = pt->G < pt->nUE + 1 ? pt->G : pt->nUE + 1;
+    return (int)((variant == RA_VARIANT_N ? 24 : 2) * g + 4);
 }
 
 extern "C" const char* ra_version(void) { return "rach_b200 0.2 (sm_100a; variants W/B, U0, N)"; }

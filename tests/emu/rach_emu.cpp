@@ -75,7 +75,18 @@ static int emu_body(const PT& pt, const RaWork& w, RaShared& s, const ref_config
         if (s.nE1) { unsigned n = s.nE1; for (int t = 0; t < NT; ++t) for (unsigned i = t; i < n; i += NT) ra_phase3b_item(pt, w, s, i); }
         unsigned n4 = (unsigned)pt.P + s.nLanders;
         for (int t = 0; t < NT; ++t) for (unsigned i = t; i < n4; i += NT) ra_phase4_item(pt, w, s, acc[t], i);
-        if (s.nSingles) { if (ra_phase5_trivial(pt, s)) s.gcAdd = (int)s.nSingles; else ra_phase5_serial(pt, w, s); }
+        if (s.nSingles) {
+            if (ra_phase5_trivial(pt, s)) s.gcAdd = (int)s.nSingles;
+            else {                                  /* the kernel's phase 5, checked against the one-thread statement */
+                RaShared ref = s;
+                ra_phase5_serial(pt, w, ref);
+                ra_phase5_warp(pt, w, s);
+                if (s.tau != ref.tau || s.noGrant != ref.noGrant) {
+                    fprintf(stderr, "emu: phase 5 tau %u/%u noGrant %u/%u at ms %d\n", s.tau, ref.tau, s.noGrant, ref.noGrant, T);
+                    return -4;
+                }
+            }
+        }
         unsigned n6 = (unsigned)pt.P + s.nLanders + s.nE1;
         for (int t = 0; t < NT; ++t) for (unsigned i = t; i < n6; i += NT) ra_phase6_item<DUMP>(job, w, s, T, i);
         if (s.nSingles) for (int t = 0; t < NT; ++t) ra_hist_clear(pt, w, s, t, NT);
@@ -116,30 +127,19 @@ static int emu_run_t(const ref_config* cfg, ref_result* res, int* perUE, int NT)
     char err[256];
     if (ra_host_validate(&p, err, sizeof err) != RA_OK) { fprintf(stderr, "emu: %s\n", err); return -1; }
 
-    RaPointDev pt; memset(&pt, 0, sizeof pt);
-    pt.nUE = p.nUE; pt.P = p.nPreamble; pt.BI = p.backoffIndicator; pt.G = p.nGrantUL;
-    pt.Wn = p.maxRarWindow; pt.M = p.maxMsg2TxCount; pt.A = p.accessTime;
-    pt.maxTime = ra_horizon_ms(&p); pt.geometry = p.geometry; pt.R = ra_host_ring(&p);
-    pt.nOcc = (pt.maxTime + pt.A - 1) / pt.A; pt.seed = p.seed;
-    ra_host_fill_point(&pt);
+    RaPointDev pt;
+    ra_host_point(&p, &pt);
     std::vector<int> arrCum(pt.nOcc);
     ra_host_arrcum(&p, arrCum.data(), pt.nOcc);
     pt.arrCum = arrCum.data();
 
-    RaWork w; w.cap = pt.nUE;
-    long long g2 = 2LL * (pt.G < pt.nUE + 1 ? pt.G : pt.nUE + 1) + 2; w.cap3 = (int)g2;
-    std::vector<uint4> bucket((size_t)pt.R * w.cap), msg3((size_t)RA_M3RING * w.cap3), landerRec(w.cap),
-        uncertain(w.cap), c3(w.cap), e1Rec(w.cap3);
-    std::vector<unsigned> landerMeta(w.cap), e1Meta(w.cap3);
-    std::vector<unsigned> singles(w.cap);
-    w.bucket = bucket.data(); w.msg3 = msg3.data(); w.landerRec = landerRec.data();
-    w.landerMeta = landerMeta.data(); w.uncertain = uncertain.data(); w.c3 = c3.data();
-    w.singles = singles.data(); w.e1Rec = e1Rec.data(); w.e1Meta = e1Meta.data();
-
+    /* the block's global workspace and dynamic shared memory, laid out as the engine lays them out */
+    RaWork w;
+    const int cap3 = ra_host_cap3(RA_VARIANT_W, &pt);
+    std::vector<uint4> work((ra_work_carve(NULL, pt.nUE, cap3, pt.R, pt.P, &w) + 15) / 16);
+    ra_work_carve(reinterpret_cast<unsigned char*>(work.data()), pt.nUE, cap3, pt.R, pt.P, &w);
     RaShared s; memset(&s, 0, sizeof s);
-    std::vector<unsigned> minPos((size_t)pt.R * pt.P);
-    w.minPos = minPos.data();
-    std::vector<uint4> smem((pt.smemBytes + 15) / 16 + 1);         /* the block's dynamic shared memory (ra_layout) */
+    std::vector<uint4> smem((pt.smemBytes + 15) / 16 + 1);
     ra_emu_smem_base = reinterpret_cast<unsigned char*>(smem.data());
 
     /* the kernel's two views of a point: runtime values, or the compile-time family of the reference defaults */
@@ -174,31 +174,23 @@ static int emu_run_n_t(const ref_config* cfg, ref_result* res, int* perUE, doubl
     p.nUE = cfg->nUE; p.distribution = 2; p.nPreamble = cfg->nPreamble;
     p.backoffIndicator = cfg->backoffIndicator; p.nGrantUL = cfg->nGrantUL;
     p.maxRarWindow = cfg->maxRarWindow; p.maxMsg2TxCount = cfg->maxMsg2TxCount;
-    p.accessTime = cfg->accessTime; p.cellRadius = cfg->cellRadius; p.seed = cfg->seed;
+    p.accessTime = cfg->accessTime; p.cellRadius = cfg->cellRadius; p.geometry = cfg->geometry; p.seed = cfg->seed;
     char err[256];
     if (ra_host_validate(&p, err, sizeof err) != RA_OK) { fprintf(stderr, "emu: %s\n", err); return -1; }
-    RaPointDev pt; memset(&pt, 0, sizeof pt);
-    pt.nUE = p.nUE; pt.P = p.nPreamble; pt.BI = p.backoffIndicator; pt.G = p.nGrantUL;
-    pt.Wn = p.maxRarWindow; pt.M = p.maxMsg2TxCount; pt.A = p.accessTime;
-    pt.maxTime = ra_horizon_ms(&p); pt.geometry = cfg->geometry ? 1 : 0; pt.R = ra_host_ring(&p);
-    pt.nOcc = (pt.maxTime + pt.A - 1) / pt.A; pt.seed = p.seed; pt.cellRadius = p.cellRadius;
-    ra_host_fill_point(&pt);
+    RaPointDev pt;
+    ra_host_point(&p, &pt);
     std::vector<int> arrCum(pt.nOcc);
     ra_host_arrcum(&p, arrCum.data(), pt.nOcc);
     pt.arrCum = arrCum.data();
 
-    RaWorkN w; w.cap = pt.nUE;
-    long long g2 = 24LL * (pt.G < pt.nUE + 1 ? pt.G : pt.nUE + 1) + 4; w.cap3 = (int)g2;
-    std::vector<uint4> bucket((size_t)pt.R * w.cap), msg3((size_t)RA_M3RING * w.cap3), zombie(w.cap);
-    std::vector<double> gain(w.cap);
-    w.bucket = bucket.data(); w.msg3 = msg3.data(); w.zombie = zombie.data(); w.gain = gain.data();
-    const size_t c = (size_t)RA_NSECT * pt.P;
-    std::vector<unsigned> cnt(c), who(c), grant(c), sPos(c), ord(c), bcount(pt.R), m3count(RA_M3RING);
-    std::vector<int> sIdx(c);
-    std::vector<double> sLg(c), sGain(c);
+    /* the block's global workspace and its tables in dynamic shared memory, laid out as the engine lays them out */
+    RaWorkN w;
+    const int cap3 = ra_host_cap3(RA_VARIANT_N, &pt);
+    std::vector<uint4> work((rn_work_carve(NULL, pt.nUE, cap3, pt.R, &w) + 15) / 16);
+    rn_work_carve(reinterpret_cast<unsigned char*>(work.data()), pt.nUE, cap3, pt.R, &w);
     RaSharedN s; memset(&s, 0, sizeof s);
-    s.cnt = cnt.data(); s.who = who.data(); s.grant = grant.data(); s.sPos = sPos.data(); s.sIdx = sIdx.data();
-    s.sLg = sLg.data(); s.sGain = sGain.data(); s.ord = ord.data(); s.bcount = bcount.data(); s.m3count = m3count.data();
+    std::vector<uint4> smem((rn_smem_bytes(pt.R, pt.P) + 15) / 16);
+    rn_carve(s, reinterpret_cast<unsigned char*>(smem.data()), pt.R, pt.P);
     RaJob job; job.pt = &pt; job.rep = (unsigned)cfg->rep; job.dump = DUMP ? perUE : NULL;
 
     for (int t = 0; t < NT; ++t) rn_job_init<DUMP>(job, s, t, NT);
@@ -254,8 +246,8 @@ extern "C" int emu_run_u0(const ref_config* cfg, ref_result* res, int* perUE, fl
     p.maxTimeMs = cfg->stopMs > 0 ? cfg->stopMs : 0;
     char err[256];
     if (ra_host_validate(&p, err, sizeof err) != RA_OK) { fprintf(stderr, "emu: %s\n", err); return -1; }
-    RaPointDev pt; memset(&pt, 0, sizeof pt);
-    ra_host_point_u0(&p, &pt);
+    RaPointDev pt;
+    ra_host_point(&p, &pt);
     std::vector<RuUE> live((size_t)pt.nUE), ph((size_t)pt.nUE);
     std::vector<int> phHead((size_t)pt.R);
     RaJob job; job.pt = &pt; job.rep = (unsigned)cfg->rep; job.dump = perUE;

@@ -135,11 +135,11 @@ def test_legacy_variant_emulated(oracle, emu):
 
 
 def test_work_list_overflow_paths(oracle, tmp_path):
-    """The per-ms work lists keep their first entries in shared memory and spill to global memory
-    (RA_LCAP / RA_UCAP / RA_SCAP in rach_core.cuh).  Built here with capacities of 3 / 2 / 2 so that
-    every run overflows them; results must not change."""
+    """The singleton scans of a ms keep their first entries in shared memory and the rest in global memory
+    (RA_SCAP in rach_core.cuh).  Built here with a capacity of 2 so that every run overflows it, and phase 5
+    (the kernel's ra_phase5_warp) and the histogram clear read past the shared-memory front; results must not change."""
     so = str(tmp_path / "librach_emu_small.so")
-    subprocess.check_call(["g++", "-O2", "-fPIC", "-shared", "-std=c++17", "-DRA_LCAP=3", "-DRA_UCAP=2", "-DRA_SCAP=2",
+    subprocess.check_call(["g++", "-O2", "-fPIC", "-shared", "-std=c++17", "-DRA_SCAP=2",
                            "-DRA_NO_POS_HINT",       # also: granted non-movers always take the search fallback (phase 6b)
                            "-I", os.path.join(ROOT, "include"), "-I", os.path.join(ROOT, "oracle"),
                            "-I", os.path.join(ROOT, "5g-nr-randomaccess_b200", "csrc"),
