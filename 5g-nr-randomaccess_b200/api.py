@@ -13,6 +13,7 @@ LIB_PATH = os.environ.get("RACH_GPU_LIB") or os.path.join(HERE, "librach_gpu.so"
 
 RA_VARIANT_W, RA_VARIANT_U0, RA_VARIANT_N = 0, 1, 2
 RA_DUMP_FIELDS = 16
+HIST_DELAY, HIST_TX, HIST_FAIL = 0, 1, 2     # RA_HIST_*: timer, preambleTxCounter, failCount of the successful UEs
 DUMP_NAMES = ["timer", "active", "txTime", "firstTxTime", "secondTxTime", "nowBackoff", "preamble",
               "preambleChange", "rarWindow", "maxRarCounter", "preambleTxCounter", "msg2Flag",
               "connectionRequest", "msg4Flag", "failCount", "sector"]
@@ -48,7 +49,7 @@ assert STATS_DTYPE.itemsize == C.sizeof(RaStats)
 
 class RaOptions(C.Structure):
     _fields_ = [("repOffset", C.c_int), ("dumpUEs", C.c_int), ("ctasPerSM", C.c_int),
-                ("phaseTimers", C.c_int), ("reserved", C.c_int * 4)]
+                ("phaseTimers", C.c_int), ("histograms", C.c_int), ("reserved", C.c_int * 3)]
 
 
 DUMP_CB = C.CFUNCTYPE(None, C.c_void_p, C.c_int, C.c_int, C.POINTER(RaStats), C.POINTER(C.c_int))
@@ -56,7 +57,7 @@ DUMP_CB = C.CFUNCTYPE(None, C.c_void_p, C.c_int, C.c_int, C.POINTER(RaStats), C.
 SYMBOLS = ["ra_sim_create", "ra_sim_create_ex", "ra_last_create_error", "ra_last_create_code", "ra_sim_run", "ra_sim_run_stream", "ra_sim_stats",
            "ra_sim_stats_all", "ra_sim_dump_ues", "ra_sim_geometry", "ra_sim_gains", "ra_sim_kernel_ms",
            "ra_sim_gpu_launches", "ra_sim_phase_cycles", "ra_sim_destroy", "ra_sim_last_error", "ra_params_default",
-           "ra_horizon_ms", "ra_arrival_schedule", "ra_params_validate", "ra_version"]
+           "ra_horizon_ms", "ra_arrival_schedule", "ra_params_validate", "ra_version", "ra_hist_bins", "ra_sim_histogram"]
 
 _lib = None
 
@@ -88,6 +89,8 @@ def load_lib():
     lib.ra_sim_dump_ues.argtypes = [vp, C.c_int, C.c_int, vp]
     lib.ra_sim_geometry.argtypes = [vp, C.c_int, C.c_int, vp]
     lib.ra_sim_gains.argtypes = [vp, C.c_int, C.c_int, vp]
+    lib.ra_sim_histogram.argtypes = [vp, C.c_int, C.c_int, vp]
+    lib.ra_hist_bins.argtypes = [C.POINTER(RaParams), C.c_int]
     lib.ra_sim_kernel_ms.restype = C.c_double
     lib.ra_sim_kernel_ms.argtypes = [vp]
     lib.ra_sim_gpu_launches.restype = C.c_longlong
@@ -124,6 +127,12 @@ def validate_params(params):
     return rc, buf.value.decode()
 
 
+def hist_bins(params, kind):
+    """Bins of histogram `kind` (HIST_*) for a point: horizon + 7 for HIST_DELAY, 256 otherwise; RA_E_INVAL (-1) for
+    an unknown kind or HIST_FAIL on variant N / U0.  Needs no device."""
+    return load_lib().ra_hist_bins(C.byref(params), kind)
+
+
 def arrival_schedule(params):
     lib = load_lib()
     h = lib.ra_horizon_ms(C.byref(params))
@@ -135,14 +144,15 @@ def arrival_schedule(params):
 class RachSim:
     """points x reps replications of the RACH state machine on the GPU(s)."""
 
-    def __init__(self, points, reps=1, devices=None, rep_offset=0, dump_ues=False, ctas_per_sm=0, phase_timers=False):
+    def __init__(self, points, reps=1, devices=None, rep_offset=0, dump_ues=False, ctas_per_sm=0, phase_timers=False,
+                 histograms=False):
         lib = load_lib()
         self._lib = lib
         self.points = list(points)
         self.reps = int(reps)
         arr = (RaParams * len(self.points))(*self.points)
         opt = RaOptions(repOffset=rep_offset, dumpUEs=1 if dump_ues else 0, ctasPerSM=ctas_per_sm,
-                        phaseTimers=1 if phase_timers else 0)
+                        phaseTimers=1 if phase_timers else 0, histograms=1 if histograms else 0)
         if devices is None:
             dev, nd = None, 0
         else:
@@ -203,6 +213,14 @@ class RachSim:
         n = self.points[point].nUE
         out = np.zeros(n, dtype=np.float64)
         self._check(self._lib.ra_sim_gains(self._h, point, rep, out.ctypes.data_as(C.c_void_p)))
+        return out
+
+    def histogram(self, point, kind):
+        """ra_sim_histogram: counts per value of `kind` (HIST_DELAY / HIST_TX / HIST_FAIL) over the UEs of `point` that
+        finished, summed over its replications and devices.  Needs histograms=True and a run."""
+        n = hist_bins(self.points[point], kind) if 0 <= point < len(self.points) else 1
+        out = np.zeros(max(n, 1), dtype=np.uint64)
+        self._check(self._lib.ra_sim_histogram(self._h, point, kind, out.ctypes.data_as(C.c_void_p)))
         return out
 
     def phase_cycles(self):

@@ -197,6 +197,7 @@ struct RaWork {
                                  register-spill working set of 5 resident blocks (measured: 10 % slower) */
     uint4*    e1Rec;          /* [cap3] Msg3 restarts that land on the current ms (W:693)   */
     unsigned* e1Meta;         /* [cap3] 1 = absorbed by a later scan                        */
+    unsigned* hist;           /* [histLen] the replication's histograms (ra_hist_add), or NULL */
     int cap, cap3;
 };
 
@@ -207,8 +208,9 @@ static inline void* ra_carve_next(unsigned char* base, size_t& off, size_t bytes
     return p;
 }
 
-/* lays out one block's workspace at `base` for a ring of R move buckets and P preambles; returns its size in bytes */
-static inline size_t ra_work_carve(unsigned char* base, int cap, int cap3, int R, int P, RaWork* w) {
+/* lays out one block's workspace at `base` for a ring of R move buckets and P preambles, with a histogram region of
+ * histLen counters (0 = none); returns its size in bytes */
+static inline size_t ra_work_carve(unsigned char* base, int cap, int cap3, int R, int P, RaWork* w, int histLen = 0) {
     const size_t c = (size_t)cap, c3 = (size_t)cap3;
     size_t off = 0;
     w->bucket = (uint4*)ra_carve_next(base, off, sizeof(uint4) * c * (size_t)R);
@@ -221,6 +223,7 @@ static inline size_t ra_work_carve(unsigned char* base, int cap, int cap3, int R
     w->e1Rec = (uint4*)ra_carve_next(base, off, sizeof(uint4) * c3);
     w->e1Meta = (unsigned*)ra_carve_next(base, off, sizeof(unsigned) * c3);
     w->minPos = (unsigned*)ra_carve_next(base, off, sizeof(unsigned) * (size_t)R * (size_t)P);
+    w->hist = histLen ? (unsigned*)ra_carve_next(base, off, sizeof(unsigned) * (size_t)histLen) : NULL;
     w->cap = cap; w->cap3 = cap3;
     return off;
 }
@@ -241,13 +244,45 @@ struct RaShared {
 /* per-thread counters, folded into RaShared at the end of the replication */
 struct RaAcc { unsigned contFailed, collP, txop, collScans, totScans; };
 
+/* the histogram region a job starts with: none on the device (the kernels set it); in the host emulation the caller's
+ * (NULL: none), as with ra_emu_smem_base */
+#ifdef __CUDA_ARCH__
+#define RA_JOB_HIST0 nullptr
+#else
+static thread_local unsigned* ra_emu_hist_base;
+#define RA_JOB_HIST0 ra_emu_hist_base
+#endif
+
 template <class PT>
 struct RaJobT {
     const PT* pt;             /* RaPointDev, or a compile-time view of it (RaPointDef)      */
     unsigned rep;             /* tape replication id                                        */
     int* dump;                /* [nUE][16] or NULL                                          */
+    unsigned* hist = RA_JOB_HIST0;   /* the block's (U0: the warp's) histogram region, or NULL */
 };
 typedef RaJobT<RaPointDev> RaJob;
+
+/* ---- histograms of the successful UEs (ra_options.histograms) ----------------------------
+ * A point's region holds three histograms back to back, 32-bit counters (a replication has fewer than 2^24 successes):
+ *   [0, maxTime + 7)   delay: timer at success in ms.  W and N record T - timerStart + 6 with T < maxTime (W:674,
+ *                      N:504-508), U0's timer is at most maxTime: so 0 .. maxTime + 6
+ *   [+0, +256)         preambleTxCounter (N: nTxPreamble), the last bin counts 255 and above
+ *   [+256, +512)       failCount (W/B only; N and U0 pass 0 and that part is never reported) */
+#define RA_HIST_TOP 256
+RA_HD int ra_hist_delay_bins(int maxTime) { return maxTime + 7; }
+RA_HD int ra_hist_len(int maxTime) { return maxTime + 7 + 2 * RA_HIST_TOP; }
+
+/* the success event of one UE (W:720-728 / N:504-508 / U0:113-115) */
+template <class PT>
+RA_HD void ra_hist_add(const RaJobT<PT>& job, unsigned delay, unsigned tx, unsigned fail) {
+    unsigned* h = job.hist;
+    if (!h) return;
+    const unsigned nD = (unsigned)ra_hist_delay_bins(job.pt->maxTime);
+    /* the clamps keep the adds in the region; the delay bound above makes its clamp unreachable */
+    RA_AADD(&h[delay < nD ? delay : nD - 1u], 1u);
+    RA_AADD(&h[nD + (tx < RA_HIST_TOP - 1u ? tx : RA_HIST_TOP - 1u)], 1u);
+    RA_AADD(&h[nD + RA_HIST_TOP + (fail < RA_HIST_TOP - 1u ? fail : RA_HIST_TOP - 1u)], 1u);
+}
 
 /* ---- record packing ---------------------------------------------------------------------- */
 /* x: idx   y: txTime   z: timerStart | failCount<<16   w: preamble | mrc<<8 | ptc<<16 | flag<<31
@@ -598,6 +633,7 @@ RA_HD int ra_msg3_item(const RaJobT<PT>& job, const RaWork& w, RaShared& s, RaAc
             RA_AADD64(&s.txSum, ra_rec_ptc(rec));
             RA_AADD64(&s.delaySum, timer);
             RA_AADD64(&s.failSum, ra_rec_fail(rec));
+            ra_hist_add(job, timer, ra_rec_ptc(rec), ra_rec_fail(rec));
             if (DUMP) {
                 int* row = job.dump + (size_t)idx * RA_DUMP_W;
                 row[0] = (int)timer; row[1] = 0; row[2] = T; row[5] = 0;

@@ -67,17 +67,20 @@ struct RaWorkN {
     uint4*  msg3;        /* [RA_M3RING][cap3]                                                */
     uint4*  zombie;      /* [cap]  restarts that can never transmit again (dump only)        */
     double* gain;        /* [cap]  channelGain of every arrived UE (N:191)                   */
+    unsigned* hist;      /* [histLen] the replication's histograms (ra_hist_add), or NULL    */
     int cap, cap3;
 };
 
-/* lays out one block's workspace at `base` for a ring of R buckets; returns its size in bytes (ra_work_carve) */
-static inline size_t rn_work_carve(unsigned char* base, int cap, int cap3, int R, RaWorkN* w) {
+/* lays out one block's workspace at `base` for a ring of R buckets and histLen histogram counters (0 = none); returns its
+ * size in bytes (ra_work_carve) */
+static inline size_t rn_work_carve(unsigned char* base, int cap, int cap3, int R, RaWorkN* w, int histLen = 0) {
     const size_t c = (size_t)cap, c3 = (size_t)cap3;
     size_t off = 0;
     w->bucket = (uint4*)ra_carve_next(base, off, sizeof(uint4) * c * (size_t)R);
     w->msg3 = (uint4*)ra_carve_next(base, off, sizeof(uint4) * c3 * RA_M3RING);
     w->zombie = (uint4*)ra_carve_next(base, off, sizeof(uint4) * c);
     w->gain = (double*)ra_carve_next(base, off, sizeof(double) * c);
+    w->hist = histLen ? (unsigned*)ra_carve_next(base, off, sizeof(unsigned) * (size_t)histLen) : NULL;
     w->cap = cap; w->cap3 = cap3;
     return off;
 }
@@ -408,6 +411,7 @@ RA_HD void rn_msg3_item(const RaJob& job, const RaWorkN& w, RaSharedN& s, int T,
             RA_AADD(&s.nSuccess, 1u);
             RA_AADD64(&s.txSum, rn_ntx(r));
             RA_AADD64(&s.delaySum, timer);
+            ra_hist_add(job, timer, rn_ntx(r), 0u);                /* N has no failCount */
             if (DUMP) {
                 int* row = job.dump + (size_t)idx * RA_DUMP_W;
                 row[0] = (int)timer; row[1] = 0; row[2] = T; row[5] = 0; row[6] = (int)rn_p(r); row[8] = 0;

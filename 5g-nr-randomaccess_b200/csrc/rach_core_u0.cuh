@@ -38,9 +38,10 @@ struct RU_ALIGN RuUE {   /* 64 bytes; the first 16 are all a collision scan read
 };
 
 /* RuUE entries of one replication's global workspace: live-list overflow [cap], phantom store [cap], phantom calendar
- * heads [maxR ints] */
-RA_HD size_t ru_work_elems(int cap, int maxR) {
-    return 2 * (size_t)cap + ((size_t)maxR * sizeof(int) + sizeof(RuUE) - 1) / sizeof(RuUE);
+ * heads [maxR ints], histogram region [histLen unsigned] (0 = none) */
+RA_HD size_t ru_work_elems(int cap, int maxR, int histLen = 0) {
+    return 2 * (size_t)cap + ((size_t)maxR * sizeof(int) + sizeof(RuUE) - 1) / sizeof(RuUE)
+         + ((size_t)histLen * sizeof(unsigned) + sizeof(RuUE) - 1) / sizeof(RuUE);
 }
 
 struct RuStats { int simTime, nSuccess; long long txSum, delaySum, collisionPreambles, totalPreambleTxop, dropped; int overflow; };
@@ -178,6 +179,7 @@ RA_HD void ru_serial_ms(const RaJob& job, RuUE* live, RuUE* win, int winCap, RuU
         r.nSuccess += ru_msg3_timer(job, u, time, k);
         if (u.msg4Flag == 1) {
             st.txSum += u.preambleTxCounter; st.delaySum += u.timer; nGone++;
+            ra_hist_add(job, (unsigned)u.timer, (unsigned)u.preambleTxCounter, 0u);   /* U0 has no failCount */
             if (DUMP) ru_dump_row(job.dump + (size_t)u.idx * RA_DUMP_W, u);
             u.active = -2;
         } else if (u.raFailed == -1) {                                    /* frozen from now on: to the phantom calendar */
@@ -267,6 +269,7 @@ RW_FN void ru_warp_ms(const RaJob& job, RuUE* win, RuUE* ph, int* phHead, int ca
             keep[l] = !fin[l] && !drp[l];
             if (fin[l]) {
                 sm.txSum[l] += u[l].preambleTxCounter; sm.delaySum[l] += u[l].timer;
+                ra_hist_add(job, (unsigned)u[l].timer, (unsigned)u[l].preambleTxCounter, 0u);
                 if (DUMP) ru_dump_row(job.dump + (size_t)u[l].idx * RA_DUMP_W, u[l]);
             }
         }

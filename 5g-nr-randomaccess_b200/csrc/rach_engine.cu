@@ -77,9 +77,22 @@ struct RaKernelArgs {
     int*              errFlag;
     volatile int*     doneFlags;    /* [nJobs] host-mapped: 1 = the replication's stats and dump rows are complete (streaming), or NULL */
     ra_u64*           phaseCycles;  /* [RA_NPHASE] cycles of thread 0 per phase, summed over blocks */
+    ra_u64*           histSum;      /* [nPoints][histLen] histograms per point, summed over replications, or NULL */
     size_t            dumpStride;
     int               nJobs, maxP, maxR;
+    int               histLen;      /* counters of a block's histogram region (0 = histograms off) */
 };
+
+/* End of a replication, after the barrier that ends it: the block's non-zero bins are added to the point's sums and the
+ * region is zeroed for the block's next replication (whose first add follows the barriers that start it).  Shared by the
+ * three kernels; the region and the point's sums have the layout of ra_hist_add. */
+__device__ __forceinline__ void ra_hist_flush(unsigned* h, int maxTime, ra_u64* out, int tid, int nt) {
+    const int n = ra_hist_len(maxTime);
+    for (int i = tid; i < n; i += nt) {
+        const unsigned v = h[i];
+        if (v) { atomicAdd(&out[i], (ra_u64)v); h[i] = 0; }
+    }
+}
 
 template <bool DUMP, int NT, int MINB, bool FIXED, bool TIMERS = false>
 __global__ void __launch_bounds__(NT, MINB) ra_step_kernel(RaKernelArgs a) {
@@ -112,6 +125,7 @@ __global__ void __launch_bounds__(NT, MINB) ra_step_kernel(RaKernelArgs a) {
         const PT& pt = static_cast<const PT&>(sPt);
         RaJobT<PT> job; job.pt = &pt; job.rep = a.jobRep[jobId];
         job.dump = DUMP ? a.dump + (size_t)jobId * a.dumpStride : nullptr;
+        job.hist = w.hist;
         ra_job_init<DUMP>(job, s, tid, nt);
         RaAcc acc; acc.contFailed = acc.collP = acc.txop = acc.collScans = acc.totScans = 0;
         __syncthreads();
@@ -260,6 +274,7 @@ __global__ void __launch_bounds__(NT, MINB) ra_step_kernel(RaKernelArgs a) {
         if (acc.collScans) atomicAdd(&s.collScans, (ra_u64)acc.collScans);
         if (acc.totScans) atomicAdd(&s.totScans, (ra_u64)acc.totScans);
         __syncthreads();
+        if (w.hist) ra_hist_flush(w.hist, pt.maxTime, a.histSum + (size_t)a.jobPoint[jobId] * a.histLen, tid, nt);
         if (tid == 0) {
             ra_stats st; memset(&st, 0, sizeof st);
             st.simTimeMs = simTime; st.nSuccess = (int)s.nSuccess;
@@ -302,6 +317,7 @@ __global__ void __launch_bounds__(RA_NT_N, RA_MINB_N) ra_step_kernel_n(RaKernelA
         const RaPointDev& pt = sPt;
         RaJob job; job.pt = &pt; job.rep = a.jobRep[jobId];
         job.dump = DUMP ? a.dump + (size_t)jobId * a.dumpStride : nullptr;
+        job.hist = w.hist;
         rn_job_init<DUMP>(job, s, tid, nt);
         __syncthreads();
         int simTime = pt.maxTime;
@@ -339,6 +355,7 @@ __global__ void __launch_bounds__(RA_NT_N, RA_MINB_N) ra_step_kernel_n(RaKernelA
             }
         }
         __syncthreads();
+        if (w.hist) ra_hist_flush(w.hist, pt.maxTime, a.histSum + (size_t)a.jobPoint[jobId] * a.histLen, tid, nt);
         const int last = simTime < pt.maxTime ? simTime : pt.maxTime - 1;
         if (DUMP) {
             rn_dump_inflight(job, w, s, last, tid, nt);
@@ -372,14 +389,17 @@ static size_t ru_smem_bytes(int maxR, bool headsInSmem) {
     return RU_WIN * sizeof(RuUE) + (headsInSmem ? (size_t)maxR * sizeof(int) : 0);
 }
 
-/* one warp (= one block) per replication; lanesOn = 0 runs the serial step on lane 0 in every ms */
-template <bool DUMP>
+/* one warp (= one block) per replication; lanesOn = 0 runs the serial step on lane 0 in every ms.  HIST: histograms on --
+ * a template parameter here (the step kernels test w.hist at run time instead) because the live pointer cost
+ * this kernel a register, past the 120 of the allocation step */
+template <bool DUMP, bool HIST>
 __global__ void __launch_bounds__(32) ra_u0_kernel(RaKernelArgs a, int cap, int headsInSmem, int lanesOn) {
     extern __shared__ __align__(16) unsigned char ru_dyn_smem[];
     const int lane = threadIdx.x;
-    RuUE* live = a.liveBase + (size_t)blockIdx.x * ru_work_elems(cap, a.maxR);
+    RuUE* live = a.liveBase + (size_t)blockIdx.x * ru_work_elems(cap, a.maxR, HIST ? a.histLen : 0);
     RuUE* ph = live + cap;
     int* phHead = reinterpret_cast<int*>(ph + cap);
+    unsigned* hist = HIST ? reinterpret_cast<unsigned*>(live + ru_work_elems(cap, a.maxR, 0)) : nullptr;
     RuUE* win = reinterpret_cast<RuUE*>(ru_dyn_smem);
     if (headsInSmem) phHead = reinterpret_cast<int*>(ru_dyn_smem + RU_WIN * sizeof(RuUE));
     for (;;) {
@@ -390,9 +410,14 @@ __global__ void __launch_bounds__(32) ra_u0_kernel(RaKernelArgs a, int cap, int 
         const RaPointDev* pt = &a.points[a.jobPoint[jobId]];
         RaJob job; job.pt = pt; job.rep = a.jobRep[jobId];
         job.dump = DUMP ? a.dump + (size_t)jobId * a.dumpStride : nullptr;
+        job.hist = hist;
         RuStats st;
         ru_run_replication<DUMP>(job, live, win, RU_WIN, ph, phHead, cap, lanesOn, &st);
         __syncwarp();
+        if (HIST) {
+            ra_hist_flush(hist, pt->maxTime, a.histSum + (size_t)a.jobPoint[jobId] * a.histLen, lane, 32);
+            __syncwarp();
+        }
         if (lane != 0) continue;
         ra_stats o; memset(&o, 0, sizeof o);
         o.simTimeMs = st.simTime; o.nSuccess = st.nSuccess; o.preambleTxSum = st.txSum; o.delaySum = st.delaySum;
@@ -444,6 +469,9 @@ struct RaDev {
     ra_stats* dStats = nullptr; RaWork* dWorks = nullptr; RaWorkN* dWorksN = nullptr; unsigned char* dWorkspace = nullptr;
     double* dGainDump = nullptr;
     int* dDump = nullptr; int* dErr = nullptr; float* dGeom = nullptr; ra_u64* dCyc = nullptr;
+    ra_u64* dHist = nullptr;          /* [nPoints][histLen] per-point histograms of this device's replications */
+    unsigned char* histRegion = nullptr; size_t histPitch = 0;   /* block 0's histogram region; the next block's is histPitch further */
+    std::vector<ra_u64> hHist;
     int grid = 0, nt = 0; size_t smem = 0; const void* kern = nullptr;
     cudaStream_t stream = nullptr; cudaEvent_t e0 = nullptr, e1 = nullptr;
     std::vector<ra_stats> hStats;
@@ -477,6 +505,8 @@ struct ra_sim {
     ra_options opt;
     std::vector<RaDev> devs;
     std::vector<ra_stats> stats;              /* [nPoints*reps] */
+    std::vector<ra_u64> hist;                 /* [nPoints][histLen], summed over devices (ra_options.histograms) */
+    int histLen = 0;                          /* counters per point and per block region; 0 = histograms off */
     std::vector<int> jobDev, jobLocal;        /* where each global job ran */
     bool ran = false;
     double kernelMs = 0; long long launches = 0;
@@ -498,7 +528,7 @@ static void ra_free_dev(RaDev& d) {
     for (int* p : d.dArrCum) cudaFree(p);
     cudaFree(d.dPoints); cudaFree(d.dJobPoint); cudaFree(d.dJobRep); cudaFree(d.dCounter);
     cudaFree(d.dStats); cudaFree(d.dWorks); cudaFree(d.dWorkspace); cudaFree(d.dDump); cudaFree(d.dErr);
-    cudaFree(d.dGeom); cudaFree(d.dCyc); cudaFree(d.dWorksN); cudaFree(d.dGainDump);
+    cudaFree(d.dGeom); cudaFree(d.dCyc); cudaFree(d.dWorksN); cudaFree(d.dGainDump); cudaFree(d.dHist);
     if (d.e0) cudaEventDestroy(d.e0);
     if (d.e1) cudaEventDestroy(d.e1);
     if (d.stream) cudaStreamDestroy(d.stream);
@@ -546,12 +576,16 @@ static int ra_setup_device(ra_sim* sim, RaDev& d) {
         cudaError_t e = cudaMalloc(&d.dDump, bytes);
         if (e != cudaSuccess) { sim->err = "dump buffer does not fit on the device (dumpUEs keeps nUE*16 ints per replication)"; return RA_E_NOMEM; }
     }
+    if (sim->histLen) {
+        RA_CUDA(sim, cudaMalloc(&d.dHist, sizeof(ra_u64) * (size_t)sim->histLen * sim->nPoints));
+        d.hHist.resize((size_t)sim->histLen * sim->nPoints);
+    }
 
     if (sim->variant == RA_VARIANT_U0) {
         /* one warp (block) per replication; global live-list overflow + phantom store of cap UEs (64 B each) per block */
         size_t freeB = 0, totalB = 0;
         RA_CUDA(sim, cudaMemGetInfo(&freeB, &totalB));
-        const size_t perThread = sizeof(RuUE) * ru_work_elems(sim->cap, sim->maxR);
+        const size_t perThread = sizeof(RuUE) * ru_work_elems(sim->cap, sim->maxR, sim->histLen);
         long long threads = std::min<long long>(nJobs, (long long)((double)freeB * 0.85 / (double)perThread));
         threads = std::min<long long>(threads, (long long)prop.multiProcessorCount * 32);   /* resident blocks */
         if (threads < 1) { sim->err = "not enough device memory for one U0 live list"; return RA_E_NOMEM; }
@@ -559,6 +593,10 @@ static int ra_setup_device(ra_sim* sim, RaDev& d) {
         d.smem = 0;
         cudaError_t e = cudaMalloc(&d.dWorkspace, perThread * (size_t)d.grid);
         if (e != cudaSuccess) { sim->err = std::string("U0 workspace cudaMalloc failed: ") + cudaGetErrorString(e); return RA_E_NOMEM; }
+        if (sim->histLen) {
+            d.histRegion = d.dWorkspace + sizeof(RuUE) * ru_work_elems(sim->cap, sim->maxR, 0);
+            d.histPitch = perThread;
+        }
         return RA_OK;
     }
     /* grid and per-block workspace */
@@ -611,8 +649,8 @@ static int ra_setup_device(ra_sim* sim, RaDev& d) {
     }
 
     RaWork sizeW; RaWorkN sizeN;
-    const size_t perBlock = isN ? rn_work_carve(nullptr, sim->cap, sim->cap3, sim->maxR, &sizeN)
-                                : ra_work_carve(nullptr, sim->cap, sim->cap3, sim->maxR, sim->maxP, &sizeW);
+    const size_t perBlock = isN ? rn_work_carve(nullptr, sim->cap, sim->cap3, sim->maxR, &sizeN, sim->histLen)
+                                : ra_work_carve(nullptr, sim->cap, sim->cap3, sim->maxR, sim->maxP, &sizeW, sim->histLen);
 
     size_t freeB = 0, totalB = 0;
     RA_CUDA(sim, cudaMemGetInfo(&freeB, &totalB));
@@ -627,13 +665,15 @@ static int ra_setup_device(ra_sim* sim, RaDev& d) {
     }
     if (isN) {
         std::vector<RaWorkN> worksN(grid);
-        for (int b = 0; b < grid; ++b) rn_work_carve(d.dWorkspace + perBlock * (size_t)b, sim->cap, sim->cap3, sim->maxR, &worksN[b]);
+        for (int b = 0; b < grid; ++b) rn_work_carve(d.dWorkspace + perBlock * (size_t)b, sim->cap, sim->cap3, sim->maxR, &worksN[b], sim->histLen);
+        d.histRegion = (unsigned char*)worksN[0].hist; d.histPitch = perBlock;
         RA_CUDA(sim, cudaMalloc(&d.dWorksN, sizeof(RaWorkN) * grid));
         RA_CUDA(sim, cudaMemcpy(d.dWorksN, worksN.data(), sizeof(RaWorkN) * grid, cudaMemcpyHostToDevice));
         return RA_OK;
     }
     std::vector<RaWork> works(grid);
-    for (int b = 0; b < grid; ++b) ra_work_carve(d.dWorkspace + perBlock * (size_t)b, sim->cap, sim->cap3, sim->maxR, sim->maxP, &works[b]);
+    for (int b = 0; b < grid; ++b) ra_work_carve(d.dWorkspace + perBlock * (size_t)b, sim->cap, sim->cap3, sim->maxR, sim->maxP, &works[b], sim->histLen);
+    d.histRegion = (unsigned char*)works[0].hist; d.histPitch = perBlock;
     RA_CUDA(sim, cudaMalloc(&d.dWorks, sizeof(RaWork) * grid));
     RA_CUDA(sim, cudaMemcpy(d.dWorks, works.data(), sizeof(RaWork) * grid, cudaMemcpyHostToDevice));
     return RA_OK;
@@ -683,7 +723,9 @@ extern "C" ra_sim* ra_sim_create_ex(const ra_params* points, int nPoints, int re
         sim->cap = std::max(sim->cap, pt.nUE);
         sim->cap3 = std::max(sim->cap3, ra_host_cap3(p.variant, &pt));
         sim->dumpStride = std::max(sim->dumpStride, (size_t)pt.nUE * RA_DUMP_W);
+        if (sim->opt.histograms) sim->histLen = std::max(sim->histLen, ra_hist_len(pt.maxTime));
     }
+    sim->hist.assign((size_t)sim->histLen * nPoints, 0);
     /* the engines index a block's move calendar with 32 bits (ring x capacity records of 16 bytes: 64 GB) */
     if ((unsigned long long)sim->maxR * (unsigned long long)sim->cap >= (1ull << 32)) {
         g_createErr = "ring x nUE exceeds 2^32 calendar records per replication"; g_createCode = RA_E_INVAL; delete sim; return nullptr;
@@ -730,10 +772,16 @@ static int ra_launch_device(ra_sim* sim, RaDev& d, bool stream = false) {
     RA_CUDA(sim, cudaMemsetAsync(d.dCounter, 0, sizeof(unsigned), d.stream));
     RA_CUDA(sim, cudaMemsetAsync(d.dErr, 0, sizeof(int), d.stream));
     RA_CUDA(sim, cudaMemsetAsync(d.dCyc, 0, sizeof(ra_u64) * RA_NPHASE, d.stream));
+    if (sim->histLen) {
+        RA_CUDA(sim, cudaMemsetAsync(d.dHist, 0, sizeof(ra_u64) * d.hHist.size(), d.stream));
+        /* one strided memset over the regions of all blocks (a run that completes leaves them zero as well) */
+        RA_CUDA(sim, cudaMemset2DAsync(d.histRegion, d.histPitch, 0, sizeof(unsigned) * (size_t)sim->histLen, (size_t)d.grid, d.stream));
+    }
     RaKernelArgs a; memset(&a, 0, sizeof a);
     a.points = d.dPoints; a.jobPoint = d.dJobPoint; a.jobRep = d.dJobRep; a.works = d.dWorks;
     a.jobCounter = d.dCounter; a.stats = d.dStats; a.dump = d.dDump; a.errFlag = d.dErr; a.phaseCycles = sim->opt.phaseTimers ? d.dCyc : nullptr;
     a.dumpStride = sim->dumpStride; a.nJobs = nJobs; a.maxP = sim->maxP; a.maxR = sim->maxR;
+    a.histSum = d.dHist; a.histLen = sim->histLen;
     if (stream) {
         if (!d.hDone) {
             RA_CUDA(sim, cudaHostAlloc(&d.hDone, sizeof(int) * (size_t)nJobs, cudaHostAllocMapped | cudaHostAllocPortable));
@@ -753,8 +801,10 @@ static int ra_launch_device(ra_sim* sim, RaDev& d, bool stream = false) {
         const size_t sm = ru_smem_bytes(sim->maxR, heads != 0);
         const char* mode = getenv("RACH_U0");   /* RACH_U0=serial: the one-thread formulation, for cross-checks */
         const int lanesOn = !(mode && mode[0] == 's');
-        if (sim->opt.dumpUEs) ra_u0_kernel<true><<<d.grid, 32, sm, d.stream>>>(a, sim->cap, heads, lanesOn);
-        else ra_u0_kernel<false><<<d.grid, 32, sm, d.stream>>>(a, sim->cap, heads, lanesOn);
+        void (*k)(RaKernelArgs, int, int, int) =
+            sim->opt.dumpUEs ? (sim->histLen ? ra_u0_kernel<true, true> : ra_u0_kernel<true, false>)
+                             : (sim->histLen ? ra_u0_kernel<false, true> : ra_u0_kernel<false, false>);
+        k<<<d.grid, 32, sm, d.stream>>>(a, sim->cap, heads, lanesOn);
     } else {
         void* kargs[] = {&a};
         RA_CUDA(sim, cudaLaunchKernel(d.kern, dim3(d.grid), dim3(d.nt), kargs, d.smem, d.stream));
@@ -763,6 +813,8 @@ static int ra_launch_device(ra_sim* sim, RaDev& d, bool stream = false) {
     RA_CUDA(sim, cudaEventRecord(d.e1, d.stream));
     RA_CUDA(sim, cudaMemcpyAsync(d.hStats.data(), d.dStats, sizeof(ra_stats) * nJobs, cudaMemcpyDeviceToHost, d.stream));
     RA_CUDA(sim, cudaMemcpyAsync(&d.hErr, d.dErr, sizeof(int), cudaMemcpyDeviceToHost, d.stream));
+    if (sim->histLen)
+        RA_CUDA(sim, cudaMemcpyAsync(d.hHist.data(), d.dHist, sizeof(ra_u64) * d.hHist.size(), cudaMemcpyDeviceToHost, d.stream));
     return RA_OK;
 }
 
@@ -779,12 +831,14 @@ static int ra_collect_device(ra_sim* sim, RaDev& d, double* ms) {
         return RA_E_INTERNAL;
     }
     for (size_t j = 0; j < d.jobs.size(); ++j) sim->stats[d.jobs[j]] = d.hStats[j];
+    for (size_t i = 0; i < d.hHist.size(); ++i) sim->hist[i] += d.hHist[i];
     return RA_OK;
 }
 
 extern "C" int ra_sim_run(ra_sim* sim) {
     if (!sim) return RA_E_INVAL;
     sim->launches = 0; sim->ran = false;
+    std::fill(sim->hist.begin(), sim->hist.end(), 0ull);
     /* every device is launched, then every launched device is drained -- also after an error, so that no stream is
      * still writing into this handle's buffers when the caller sees the error code (and may destroy the handle) */
     int rc = RA_OK;
@@ -826,6 +880,7 @@ extern "C" int ra_sim_run_stream(ra_sim* sim, ra_dump_cb cb, void* user) {
     if (!sim || !cb) return RA_E_INVAL;
     if (!sim->opt.dumpUEs) { sim->err = "ra_sim_run_stream needs ra_options.dumpUEs = 1 at create time"; return RA_E_STATE; }
     sim->launches = 0; sim->ran = false;
+    std::fill(sim->hist.begin(), sim->hist.end(), 0ull);
     const int kSlots = 4;                                  /* staging buffers in flight per device */
     struct Slot { int* rows = nullptr; ra_stats* st = nullptr; cudaEvent_t ev = nullptr; int job = -1; };
     struct Ring { std::vector<Slot> slots; int head = 0, inflight = 0; std::vector<char> issued; };
@@ -941,6 +996,19 @@ extern "C" int ra_sim_dump_ues(ra_sim* sim, int point, int rep, int* out) {
     RA_CUDA(sim, cudaSetDevice(d.id));
     RA_CUDA(sim, cudaMemcpy(out, d.dDump + (size_t)sim->jobLocal[job] * sim->dumpStride,
                             sizeof(int) * (size_t)sim->points[point].nUE * RA_DUMP_W, cudaMemcpyDeviceToHost));
+    return RA_OK;
+}
+
+extern "C" int ra_sim_histogram(ra_sim* sim, int point, int kind, unsigned long long* out) {
+    if (!sim || !out) return RA_E_INVAL;
+    if (!sim->ran) { sim->err = "ra_sim_histogram before ra_sim_run"; return RA_E_STATE; }
+    if (!sim->opt.histograms) { sim->err = "ra_sim_histogram needs ra_options.histograms = 1 at create time"; return RA_E_STATE; }
+    if (point < 0 || point >= sim->nPoints) { sim->err = "point out of range"; return RA_E_INVAL; }
+    const int n = ra_hist_bins(&sim->points[point], kind);
+    if (n < 0) { sim->err = "unknown histogram kind, or RA_HIST_FAIL on variant N / U0 (they have no failCount)"; return n; }
+    const int nD = ra_hist_delay_bins(sim->hostPoints[point].maxTime);
+    const size_t off = kind == RA_HIST_DELAY ? 0 : (size_t)nD + (kind == RA_HIST_FAIL ? RA_HIST_TOP : 0);
+    memcpy(out, sim->hist.data() + (size_t)point * sim->histLen + off, sizeof(unsigned long long) * (size_t)n);
     return RA_OK;
 }
 

@@ -57,6 +57,16 @@ extern "C" int ra_horizon_ms(const ra_params* p) {
     return p->distribution == 1 ? 60000 : 10000;     /* W:243, W:254 */
 }
 
+extern "C" int ra_hist_bins(const ra_params* p, int kind) {
+    if (!p) return RA_E_INVAL;
+    const int h = ra_horizon_ms(p);
+    if (h < 1) return RA_E_INVAL;
+    if (kind == RA_HIST_DELAY) return ra_hist_delay_bins(h);
+    if (kind == RA_HIST_TX) return RA_HIST_TOP;
+    if (kind == RA_HIST_FAIL && p->variant == RA_VARIANT_W) return RA_HIST_TOP;
+    return RA_E_INVAL;
+}
+
 extern "C" int ra_arrival_schedule(const ra_params* p, int* arrivals, int horizon) {
     if (!p || !arrivals || horizon < 0 || p->accessTime < 1 || p->nUE < 0) return RA_E_INVAL;
     const int n = p->nUE, accessTime = p->accessTime;

@@ -24,6 +24,10 @@
  *           --binlog     per-UE logs as compact binary instead of text: <seed>_<P>_UE<nUE>_Logs.bin = 32-byte header
  *                        ("RAUELOG1", int32 nUE, nFields = 14, seed, nPreamble, 0, 0) + nUE x 14 int32, the fields
  *                        saveResult prints after Idx (W:812-819), 56 B per UE instead of ~240 B of text
+ *           --hist       per point, <P>_<nUE>_Distributions.csv in the result directory: "metric,value,count", one row per
+ *                        non-zero bin of the histograms of the successful UEs, summed over the -t seeds (built on the GPU,
+ *                        ra_sim_histogram): delay_ms (timer, W:346), preamble_tx (preambleTxCounter, W:347; 255 = 255 and
+ *                        above) and, for --format w only, fail_count (failCount, W:348; 255 = 255 and above)
  *   The per-UE logs are written WHILE the kernel runs (ra_sim_run_stream): each finished replication is copied out
  *   asynchronously and written by the host thread; the report itself is printed afterwards in the reference's order.
  *
@@ -71,9 +75,33 @@ static void usage_and_exit(void) {
     exit(-1);
 }
 
+/* --hist: <dir>/<P>_<nUE>_Distributions.csv for every point of the handle */
+static int write_distributions(ra_sim* sim, const ra_params* pts, int nNue, const char* dir, int withFail) {
+    static const char* metric[3] = {"delay_ms", "preamble_tx", "fail_count"};
+    const int kinds[3] = {RA_HIST_DELAY, RA_HIST_TX, RA_HIST_FAIL};
+    for (int k = 0; k < nNue; ++k) {
+        char path[800];
+        snprintf(path, sizeof path, "%s/%d_%d_Distributions.csv", dir, pts[k].nPreamble, pts[k].nUE);
+        FILE* fp = fopen(path, "w");
+        if (!fp) { fprintf(stderr, "rach_sim: cannot write %s: %s\n", path, strerror(errno)); return 2; }
+        fprintf(fp, "metric,value,count\n");
+        for (int m = 0; m < (withFail ? 3 : 2); ++m) {
+            const int n = ra_hist_bins(&pts[k], kinds[m]);
+            unsigned long long* h = (unsigned long long*)malloc(sizeof *h * (size_t)n);
+            if (ra_sim_histogram(sim, k, kinds[m], h) != RA_OK) {
+                fprintf(stderr, "rach_sim: %s\n", ra_sim_last_error(sim)); free(h); fclose(fp); return 2;
+            }
+            for (int v = 0; v < n; ++v) if (h[v]) fprintf(fp, "%s,%d,%llu\n", metric[m], v, h[v]);
+            free(h);
+        }
+        fclose(fp);
+    }
+    return 0;
+}
+
 /* --format u: the report of RandomAccessSimulator.c (U0:42-143 main, U0:277-345 writers), one replication per point */
 static int report_u0(const ra_params* base, const int* nueList, int nNue, const char* outdir, int writeLogs, int device,
-                     int preambleSet, int backoffSet) {
+                     int preambleSet, int backoffSet, int hist) {
     ra_params* pts = (ra_params*)calloc((size_t)nNue, sizeof *pts);
     for (int k = 0; k < nNue; ++k) {
         ra_params_default(&pts[k], RA_VARIANT_U0);                    /* U0:48-59: 64 preambles, BI 20, 60 s */
@@ -87,6 +115,7 @@ static int report_u0(const ra_params* base, const int* nueList, int nNue, const 
     mkdir(dir, 0755);
     ra_options opt; memset(&opt, 0, sizeof opt);
     opt.dumpUEs = 1;                                                  /* the delay sum is a float accumulation in UE order */
+    opt.histograms = hist;
     ra_sim* sim = ra_sim_create_ex(pts, nNue, 1, &device, 1, &opt);
     if (!sim) { fprintf(stderr, "rach_sim: %s\n", ra_last_create_error()); return 2; }
     if (ra_sim_run(sim) != RA_OK) { fprintf(stderr, "rach_sim: %s\n", ra_sim_last_error(sim)); return 2; }
@@ -151,6 +180,7 @@ static int report_u0(const ra_params* base, const int* nueList, int nNue, const 
         }
         free(ue);
     }
+    if (hist && write_distributions(sim, pts, nNue, dir, 0) != 0) return 2;
     fprintf(stderr, "rach_sim: %d points, kernel %.1f ms (%s)\n", nNue, ra_sim_kernel_ms(sim), ra_version());
     ra_sim_destroy(sim);
     free(pts);
@@ -212,7 +242,7 @@ static int is_flag(const char* a, const char* l, const char* s, const char* alia
 int main(int argc, char* argv[]) {
     ra_params base;
     ra_params_default(&base, RA_VARIANT_W);
-    int times = 1, writeLogs = 1, device = 0, grantSet = 0, preambleSet = 0, backoffSet = 0, binlog = 0;
+    int times = 1, writeLogs = 1, device = 0, grantSet = 0, preambleSet = 0, backoffSet = 0, binlog = 0, hist = 0;
     int devList[64], nDev = 0;
     char format = 'w';
     const char* outdir = ".";
@@ -223,6 +253,7 @@ int main(int argc, char* argv[]) {
         const char* a = argv[i];
         if (strcmp(a, "--no-logs") == 0) { writeLogs = 0; i -= 1; continue; }
         if (strcmp(a, "--binlog") == 0) { binlog = 1; i -= 1; continue; }
+        if (strcmp(a, "--hist") == 0) { hist = 1; i -= 1; continue; }
         const char* v = (i + 1 < argc) ? argv[i + 1] : "";      /* the reference dereferences argv[i+1] blindly (W:94) */
         if (is_flag(a, "--times", "-t", NULL)) {
             if (atoi(v) < 1) die("Simulation count must be greater than zero.");
@@ -275,7 +306,7 @@ int main(int argc, char* argv[]) {
     if (nDev == 0) devList[nDev++] = device; else device = devList[0];
     base.seed = seed64;
     if (format != 'w' && format != 'b' && format != 'n' && format != 'u') usage_and_exit();
-    if (format == 'u') return report_u0(&base, nueList, nNue, outdir, writeLogs, device, preambleSet, backoffSet);
+    if (format == 'u') return report_u0(&base, nueList, nNue, outdir, writeLogs, device, preambleSet, backoffSet, hist);
     if (format == 'b') { base.geometry = 0; if (!grantSet) base.nGrantUL = 54; }         /* B:49, B:137-145 */
     if (format == 'n') {                                                                 /* NOMA.c:41-57 */
         ra_params n; ra_params_default(&n, RA_VARIANT_N);
@@ -298,6 +329,7 @@ int main(int argc, char* argv[]) {
     for (int k = 0; k < nNue; ++k) { pts[k] = base; pts[k].nUE = nueList[k]; }
     ra_options opt; memset(&opt, 0, sizeof opt);
     opt.dumpUEs = writeLogs;
+    opt.histograms = hist;
     ra_sim* sim = ra_sim_create_ex(pts, nNue, times, devList, nDev, &opt);
     if (!sim) { fprintf(stderr, "rach_sim: %s\n", ra_last_create_error()); return 2; }
     log_ctx lc; memset(&lc, 0, sizeof lc);
@@ -379,6 +411,7 @@ int main(int argc, char* argv[]) {
 
         }
     }
+    if (hist && write_distributions(sim, pts, nNue, dir, format == 'w') != 0) return 2;   /* B has no failCount */
     fprintf(stderr, "rach_sim: %d points x %d seeds on %d device(s), kernel %.1f ms (%s)\n", nNue, times, nDev, ra_sim_kernel_ms(sim), ra_version());
     free(lc.totalDelay);
     ra_sim_destroy(sim);

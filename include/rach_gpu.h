@@ -22,6 +22,8 @@
  *                      floats of saveSimulationLog W:735-739 stay in the host
  *   ra_sim_dump_ues    the per-UE fields saveResult prints, W:809-822 (15 ints per UE)
  *   ra_sim_geometry    the activateUEs side outputs W:392-415 (never read back by W)
+ *   ra_sim_histogram   the distributions behind the means of W:346-348: per-UE timer, preambleTxCounter and
+ *                      failCount of the UEs with msg4Flag == 1, as histograms summed over replications
  *   ra_arrival_schedule  W:246-251 / W:285-287 (B:95-100 / B:127-129): UEs arriving per ms
  *
  * Conventions: plain pointers and sizes, caller-owned outputs, no exit() inside the
@@ -60,6 +62,11 @@ extern "C" {
 #define RA_E_INTERNAL   -6   /* engine self-check tripped (overflow flag)  */
 
 #define RA_DUMP_FIELDS 16    /* ints per UE written by ra_sim_dump_ues     */
+
+/* histogram kinds of ra_sim_histogram, over the UEs with msg4Flag == 1 (W:337-348, N:504-508, U0:127-139) */
+#define RA_HIST_DELAY   0    /* timer at success in ms (the quantity delaySum sums, W:346): bins 0 .. horizon + 6, exact */
+#define RA_HIST_TX      1    /* preambleTxCounter (preambleTxSum, W:347; N: nTxPreamble): 256 bins, the last counts >= 255 */
+#define RA_HIST_FAIL    2    /* failCount (failCountSum, W:348), variant W/B only: 256 bins, the last counts >= 255 */
 
 /* One parameter point == one iteration of the reference's nUE sweep (W:221). */
 typedef struct ra_params {
@@ -111,7 +118,9 @@ typedef struct ra_options {
     int ctasPerSM;      /* 0 = engine default; resident CTAs per SM of the step kernel        */
     int phaseTimers;    /* 1 = collect per-phase cycle counters (ra_sim_phase_cycles): a separate kernel instantiation
                            (costs ~2 %), W/B dynamics only, not together with dumpUEs (RA_E_INVAL) */
-    int reserved[4];
+    int histograms;     /* 1 = accumulate the RA_HIST_* histograms of every point on the device (ra_sim_histogram);
+                           combines with dumpUEs and phaseTimers */
+    int reserved[3];
 } ra_options;
 
 typedef struct ra_sim ra_sim;
@@ -143,6 +152,12 @@ int         ra_sim_dump_ues(ra_sim* sim, int point, int rep, int* out);
 /* out[nUE * 6] floats: angle, xCoordinate, yCoordinate, distance, channelGain, (float)sector
  * (W:396-415).  Requires geometry=1. */
 int         ra_sim_geometry(ra_sim* sim, int point, int rep, float* out);
+/* out[ra_hist_bins(point, kind)]: the RA_HIST_* histogram of one point over the UEs that finished (msg4Flag == 1,
+ * W:337-348), summed over the point's replications and over all devices of the handle.  Filled by ra_sim_run and
+ * ra_sim_run_stream on the GPU; the sums of a bin times its value give delaySum / preambleTxSum / failCountSum of
+ * ra_sim_stats (for TX and FAIL while the last bin is empty).  Needs ra_options.histograms = 1 and a run (RA_E_STATE);
+ * RA_E_INVAL for a bad point or kind, and for RA_HIST_FAIL on variant N or U0 (no failCount there). */
+int         ra_sim_histogram(ra_sim* sim, int point, int kind, unsigned long long* out);
 /* variant N with dumpUEs: out[nUE] doubles = channelGain (N:183-191), 0 for UEs that never arrived;
  * ra_sim_dump_ues then writes: timer active txTime firstTxTime secondTxTime nowBackoff preamble sector
  * rarWindow msg1ReTx nTxPreamble msg2 msg3Wait RA msg3Faile RaFailed (saveResultLogs order, N:577-592) */
@@ -157,6 +172,9 @@ const char* ra_sim_last_error(const ra_sim* sim);
 /* Host-side helpers (no device needed). */
 int         ra_params_default(ra_params* p, int variant);   /* W:69-88 defaults */
 int         ra_horizon_ms(const ra_params* p);              /* W:243,254 */
+/* bins of the RA_HIST_* histogram `kind` of point p: horizon + 7 for RA_HIST_DELAY, 256 for RA_HIST_TX and (variant W
+ * only) RA_HIST_FAIL; RA_E_INVAL otherwise */
+int         ra_hist_bins(const ra_params* p, int kind);
 /* the parameter checks of ra_sim_create without a device: RA_OK, or RA_E_INVAL with the reason in err[errLen]
  * (the reference checks only "> 0" style ranges in main, W:94-158; the engine adds its packing limits: nUE <= 2^24,
  * nPreamble <= 256, backoffIndicator <= 4096, RAR window <= 255, max retx <= 256, horizon <= 65535 ms, and
